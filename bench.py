@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — train-step graphs/sec (BASELINE.json metric) of the DeformContact hot path on B200.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--workload ...] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is one full training step of the everyday.json model on config C3 of BASELINE.json — ONE
@@ -20,8 +20,10 @@ gather/segmented-sum hop kernel (K1, the north_star kernel), both timed with CUD
 installable) on the host cores.
 """
 import argparse
+import ctypes
 import json
 import os
+import signal
 import statistics
 import subprocess
 import sys
@@ -66,7 +68,16 @@ def parse():
     ap.add_argument("--order", default="random", choices=["random", "morton"],
                     help="C5: node order inside each graph: as generated (spatially random: worst-case gather locality) or Morton-sorted")
     ap.add_argument("--edges", type=float, default=10e6, help="C5 sweep: number of edges")
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="C3 train step: after the timed steps write what the last one computed as DIR/<name>.npy (float32): "
+                         "loss, l1, consistency, and grad.<parameter> / param.<parameter> for every parameter after its Adam "
+                         "update (rank 0; inputs and initial weights are seeded, so runs with the same arguments compare)")
+    args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl != "ours" or args.workload != "train_c3"):
+        ap.error("--dump-outputs writes the outputs of the C3 train step (--impl ours --workload train_c3)")
+    return args
 
 
 # --------------------------------------------------------------------------- clocks
@@ -81,8 +92,12 @@ class ClockSampler:
         try:
             f = tempfile.NamedTemporaryFile("w", suffix=".csv", delete=False)
             self.path = f.name
+            # the sampler gets SIGTERM when this process ends, so a sub-benchmark that raised before stop() or a killed run
+            # leaves no nvidia-smi behind (PR_SET_PDEATHSIG = 1)
+            prctl = ctypes.CDLL(None).prctl
             self.proc = subprocess.Popen(["nvidia-smi", f"--query-gpu={self.Q}", "--format=csv,noheader,nounits", "-lms", "100",
-                                          "-i", str(self.idx)], stdout=f, stderr=subprocess.DEVNULL)
+                                          "-i", str(self.idx)], stdout=f, stderr=subprocess.DEVNULL,
+                                         preexec_fn=lambda: prctl(1, int(signal.SIGTERM)))
         except Exception:
             self.proc = None
 
@@ -234,6 +249,14 @@ def run_reference(args):
 
 
 # --------------------------------------------------------------------------- ours
+def dump_outputs(path, arrays):
+    """--dump-outputs: every tensor of ``arrays`` as ``path/<name>.npy``, float32."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    for name, t in arrays.items():
+        np.save(os.path.join(path, f"{name}.npy"), t.detach().float().cpu().numpy())
+
+
 def _peaks():
     try:
         return json.load(open(os.path.join(ROOT, "MEASURED_PEAKS.json")))
@@ -316,7 +339,7 @@ def run_ours(args):
         loss.backward()
         flat.all_reduce()
         opt.step()
-        return loss
+        return loss.detach(), l1.detach(), lc.detach()     # what CapturedTrainStep.replay returns
 
     def barrier():
         if world > 1:
@@ -324,17 +347,18 @@ def run_ours(args):
         torch.cuda.synchronize()
 
     def timed(fn, steps):
+        """-> (ms for `steps` calls of fn, what the last call returned)"""
         barrier()
         e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
         e0.record()
         for _ in range(steps):
-            fn()
+            out = fn()
         e1.record()
         barrier()
         ms = torch.tensor([e0.elapsed_time(e1)], dtype=torch.float64, device=dev)
         if world > 1:
             tdist.all_reduce(ms, op=tdist.ReduceOp.MAX)
-        return ms.item()
+        return ms.item(), out
 
     W = max(args.warmup, 3)
     # ---- device-resident arm: the captured step replayed on resident inputs (or the eager step with --step eager)
@@ -352,10 +376,14 @@ def run_ours(args):
     if rank == 0:
         sampler.start()
     l0 = lib.dc_launch_count()
-    total_ms = timed(resident, args.steps)
+    total_ms, (loss, l1, lc) = timed(resident, args.steps)
     if not use_graph:
         launches_per_step = (lib.dc_launch_count() - l0) // args.steps
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:   # before the profiling and end-to-end arms below train the model further
+        params = list(model.named_parameters())
+        dump_outputs(args.dump_outputs, {"loss": loss, "l1": l1, "consistency": lc, **{f"grad.{k}": p.grad for k, p in params},
+                                         **{f"param.{k}": p for k, p in params}})
     ms_step = total_ms / args.steps
     value = Btot / (ms_step * 1e-3)
     del runner, resident
@@ -467,11 +495,11 @@ def run_ours(args):
                 loss_host.copy_(loss.reshape(1), non_blocking=False)      # D2H read of the step's result
         else:
             def e2e_step():
-                loss = eager_step(*assemble({k: v.to(dev, non_blocking=True) for k, v in host.items()}))
-                loss_host.copy_(loss.detach().reshape(1), non_blocking=False)
+                loss = eager_step(*assemble({k: v.to(dev, non_blocking=True) for k, v in host.items()}))[0]
+                loss_host.copy_(loss.reshape(1), non_blocking=False)
         for _ in range(3):
             e2e_step()
-        e2e_ms = timed(e2e_step, args.steps) / args.steps
+        e2e_ms = timed(e2e_step, args.steps)[0] / args.steps
         e2e = {"value": Btot / (e2e_ms * 1e-3), "unit": "graphs/s", "ms_per_step": e2e_ms,
                "h2d_bytes_per_step": h2d, "d2h_bytes_per_step": 4, "inputs": "raw", "assembled_batch_equals_resident": n3_ok}
         runner = None

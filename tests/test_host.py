@@ -144,9 +144,13 @@ print("ok", rank)
 
 def test_flat_grad_allreduce_gloo_world2(tmp_path):
     """N>1 path on CPU: world_size-2 gloo; unequal shards reproduce the global-mean gradient."""
+    import socket
     script = tmp_path / "w.py"
     script.write_text(_WORKER)
-    env = dict(os.environ, DC_ROOT=ROOT, MASTER_ADDR="127.0.0.1", MASTER_PORT="29541", WORLD_SIZE="2")
+    with socket.socket() as s:      # a port nobody else on this host holds
+        s.bind(("127.0.0.1", 0))
+        port = s.getsockname()[1]
+    env = dict(os.environ, DC_ROOT=ROOT, MASTER_ADDR="127.0.0.1", MASTER_PORT=str(port), WORLD_SIZE="2")
     procs = [subprocess.Popen([sys.executable, str(script)], env=dict(env, RANK=str(r), LOCAL_RANK=str(r)),
                               stdout=subprocess.PIPE, stderr=subprocess.STDOUT, text=True) for r in range(2)]
     outs = [p.communicate(timeout=120)[0] for p in procs]

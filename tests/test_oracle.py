@@ -235,7 +235,19 @@ def test_attn_group_equals_minibatches():
     assert_close(full, torch.cat(parts), what="attn_group vs mini-batches")
 
 
-def test_train_step_restatement_vs_reference_training_loop(golden_dir):
+@pytest.fixture
+def fixture_threads():
+    """train_loop.pt was written with 8 intra-op threads on an AVX-512 CPU.  How the fp32 products and reductions of the loop
+    are split over threads decides their last bits, and Adam's first steps (m / sqrt(v)) turn a last-bit difference in a
+    near-zero gradient into a weight difference above the elementwise bar of the test; with the same split the loop reproduces
+    the fixture bit for bit on any such CPU, whatever its core count."""
+    threads = torch.get_num_threads()
+    torch.set_num_threads(8)
+    yield
+    torch.set_num_threads(threads)
+
+
+def test_train_step_restatement_vs_reference_training_loop(golden_dir, fixture_threads):
     """The oracle's train step (oracle.train_step_loss + Adam, what every GPU train-step parity test compares against)
     reproduces the reference's OWN loop: train.py:train(config) executed unmodified for one epoch over three mini-batches
     (tests/golden/make_golden_train.py -> train_loop.pt): the three logged losses of every step, the validation loss
