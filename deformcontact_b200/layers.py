@@ -5,7 +5,7 @@ state-dict keys as torch_geometric 2.5.2, so they slot into the reference's
 ``GraphNet.__init__`` / ``forward`` (models/model.py:39-50, 69-78) and load its checkpoints
 (train.py:125, eval.py:36,89).  Forward and backward run entirely in libdcb200 (hand-written
 sm_100a CUDA reached through the C ABI); every layer is ONE registered custom op with a registered
-autograd formula (``torch.ops.dcb200.{tag_conv, gcn_conv, gat_conv, mpnn_layer}``, torch_ops.py) — the
+autograd formula (``torch.ops.dcb200.{tag_conv, gcn_conv, gat_conv / gat_conv_heads, mpnn_layer}``, torch_ops.py) — the
 modules below only hold the parameters and call the op.
 
 ``edge_index`` may be the usual ``int64 [2, E]`` tensor (the CSR pair is built once per tensor
@@ -122,25 +122,38 @@ class GCNConv(nn.Module):
 
 # ------------------------------------------------------------------------------- GATConv
 class GATConv(nn.Module):
-    """PyG 2.5.x ``GATConv(in, out)`` defaults (heads=1, concat, slope 0.2, add_self_loops);
-    keys ``lin.weight``, ``att_src``, ``att_dst``, ``bias``."""
+    """PyG 2.5.x ``GATConv(in, out, heads=1, concat=True, negative_slope=0.2, bias=True)`` with ``add_self_loops=True`` and
+    ``dropout=0``; keys ``lin.weight [H*C, in]``, ``att_src`` / ``att_dst [1, H, C]``, ``bias [H*C]`` (concat) or ``[C]`` (mean).
 
-    def __init__(self, in_channels, out_channels, heads=1, negative_slope=0.2, bias=True, precision=ops.GEMM_AUTO):
+    ``heads == 1`` runs ``torch.ops.dcb200.gat_conv`` (scores, softmax, then the K1 aggregation).  ``heads > 1`` runs
+    ``torch.ops.dcb200.gat_conv_heads``: per-head softmax and aggregation in one launch with the concat / mean epilogue
+    (``dc_gat_aggregate``), backward by receiver then by source (``dc_gat_bwd_edge_heads``, ``dc_gat_scatter_heads``).
+    Attention dropout, ``add_self_loops=False``, ``fill_value`` and ``edge_dim`` are not supported and raise."""
+
+    def __init__(self, in_channels, out_channels, heads=1, concat=True, negative_slope=0.2, bias=True, precision=ops.GEMM_AUTO, *,
+                 dropout=0.0, add_self_loops=True, edge_dim=None, fill_value="mean"):
         super().__init__()
-        if heads != 1:
-            raise NotImplementedError("GATConv: the reference constructs heads=1 (models/model.py:45); heads>1 unsupported")
+        if heads < 1:
+            raise ValueError(f"GATConv: heads must be >= 1, got {heads}")
+        if dropout != 0.0 or not add_self_loops or edge_dim is not None or fill_value != "mean":
+            raise NotImplementedError("GATConv: attention dropout, add_self_loops=False, fill_value and edge_dim are not supported")
         self.in_channels, self.out_channels, self.heads, self.negative_slope = in_channels, out_channels, heads, negative_slope
+        self.concat = concat
         self.lin = _Lin(in_channels, heads * out_channels, init="glorot")
         self.att_src = nn.Parameter(torch.empty(1, heads, out_channels))
         self.att_dst = nn.Parameter(torch.empty(1, heads, out_channels))
         _glorot_(self.att_src)
         _glorot_(self.att_dst)
-        self.bias = nn.Parameter(torch.zeros(heads * out_channels)) if bias else None
+        self.bias = nn.Parameter(torch.zeros(heads * out_channels if concat else out_channels)) if bias else None
         self.precision = precision
 
     def forward(self, x, edge_index, relu=False, ptr=None):
-        return torch.ops.dcb200.gat_conv(x, _edge_tensor(edge_index), self.lin.weight, self.att_src, self.att_dst, self.bias,
-                                         float(self.negative_slope), relu, self.precision, ptr)[0]
+        if self.heads == 1:     # the mean over one head is that head: concat and mean are the same layer
+            return torch.ops.dcb200.gat_conv(x, _edge_tensor(edge_index), self.lin.weight, self.att_src, self.att_dst, self.bias,
+                                             float(self.negative_slope), relu, self.precision, ptr)[0]
+        return torch.ops.dcb200.gat_conv_heads(x, _edge_tensor(edge_index), self.lin.weight, self.att_src, self.att_dst, self.bias,
+                                               float(self.negative_slope), self.heads, bool(self.concat), relu, self.precision,
+                                               ptr)[0]
 
 
 # ------------------------------------------------------------------------------- MPNN (A9 extension)

@@ -1032,3 +1032,60 @@ def segment_sum(rowptr, eid, val, init, N):
     out = torch.empty(N, dtype=_f32, device=val.device)
     _abi.call("dc_segment_sum", _ptr(rowptr), _ptr(eid), _ptr(val), _ptr(init), N, _ptr(out), _stream())
     return out
+
+
+# ----------------------------------------------------------------------------- K6 multi-head (csrc/gat.cu)
+def _dout_heads(heads, C_, concat):
+    """(head stride, scale) of the per-head output gradient: concat reads head h's column slice, mean reads dout / H
+    (stride 0) without materialising it."""
+    return (C_, 1.0) if concat else (0, 1.0 / heads)
+
+
+def gat_aggregate(g, xs, a_src, a_dst, slope, heads, C_, concat, bias=None, relu=False):
+    """Per-head softmax + aggregation + concat / mean + bias (+ReLU) -> (out, alpha_e [max(E,1), H], alpha_s [N, H]);
+    see dc_gat_aggregate."""
+    _need(xs, _f32, "xs"), _need(bias, _f32, "bias")
+    out = torch.empty((g.N, heads * C_ if concat else C_), dtype=_f32, device=xs.device)
+    alpha_e = torch.zeros((max(g.E, 1), heads), dtype=_f32, device=xs.device)
+    alpha_s = torch.empty((g.N, heads), dtype=_f32, device=xs.device)
+    _abi.call("dc_gat_aggregate", _ptr(g.rowptr), _ptr(g.nbr), _ptr(g.eid), _ptr(xs), _rows(xs, "xs"), _ptr(a_src), _ptr(a_dst),
+              float(slope), int(heads), int(C_), int(bool(concat)), _ptr(bias), int(bool(relu)), g.N, _ptr(out), _rows(out, "out"),
+              _ptr(alpha_e), _ptr(alpha_s), _stream())
+    return out, alpha_e, alpha_s
+
+
+def gat_bwd_edge_heads(g, a_src, a_dst, slope, alpha_e, alpha_s, xs, dout, heads, C_, concat):
+    """-> (dz_e [max(E,1), H], dz_s [N, H], da_dst [N, H]); see dc_gat_bwd_edge_heads."""
+    hs, scale = _dout_heads(heads, C_, concat)
+    dz_e = torch.zeros((max(g.E, 1), heads), dtype=_f32, device=xs.device)
+    dz_s = torch.empty((g.N, heads), dtype=_f32, device=xs.device)
+    da_dst = torch.empty((g.N, heads), dtype=_f32, device=xs.device)
+    _abi.call("dc_gat_bwd_edge_heads", _ptr(g.rowptr), _ptr(g.nbr), _ptr(g.eid), _ptr(a_src), _ptr(a_dst), float(slope),
+              _ptr(alpha_e), _ptr(alpha_s), _ptr(xs), _rows(xs, "xs"), _ptr(dout), _rows(dout, "dout"), hs, scale, int(heads),
+              int(C_), g.N, _ptr(dz_e), _ptr(dz_s), _ptr(da_dst), _stream())
+    return dz_e, dz_s, da_dst
+
+
+def gat_scatter_heads(g, alpha_e, alpha_s, dz_e, dz_s, da_dst, att_src, att_dst, dout, heads, C_, concat):
+    """-> (dxs [N, H*C], da_src [N, H]) over the by-source structure; see dc_gat_scatter_heads."""
+    hs, scale = _dout_heads(heads, C_, concat)
+    rpt, nbt, eidt = g.t
+    att_src, att_dst = att_src.contiguous(), att_dst.contiguous()
+    dxs = torch.empty((g.N, heads * C_), dtype=_f32, device=dout.device)
+    da_src = torch.empty((g.N, heads), dtype=_f32, device=dout.device)
+    _abi.call("dc_gat_scatter_heads", _ptr(rpt), _ptr(nbt), _ptr(eidt), _ptr(alpha_e), _ptr(alpha_s), _ptr(dz_e), _ptr(dz_s),
+              _ptr(da_dst), _ptr(att_src), _ptr(att_dst), _ptr(dout), _rows(dout, "dout"), hs, scale, int(heads), int(C_), g.N,
+              _ptr(dxs), _rows(dxs, "dxs"), _ptr(da_src), _stream())
+    return dxs, da_src
+
+
+def gat_att_grad(xs, da_src, da_dst, heads, C_):
+    """-> (datt_src [H*C], datt_dst [H*C]); see dc_gat_att_grad."""
+    N = xs.shape[0]
+    datt_src = torch.empty(heads * C_, dtype=_f32, device=xs.device)
+    datt_dst = torch.empty(heads * C_, dtype=_f32, device=xs.device)
+    nb = _abi.lib().dc_gat_att_grad_workspace_bytes(N, heads, C_)
+    ws = _workspace(nb, xs.device)
+    _abi.call("dc_gat_att_grad", _ptr(xs), _rows(xs, "xs"), _ptr(da_src), _ptr(da_dst), N, int(heads), int(C_), _ptr(datt_src),
+              _ptr(datt_dst), _ptr(ws), nb, _stream())
+    return datt_src, datt_dst

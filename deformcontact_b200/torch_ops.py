@@ -7,7 +7,7 @@ autograd formula whose backward is again a ``dcb200`` op.  This file holds the O
 four layers' forward / backward; the ``nn.Module``s in ``layers.py`` call these ops and nothing else.
 
     csr_build, propagate, linear, knn_table, radius_table, knn_graph, radius_graph,
-    tag_conv(+_backward), gcn_conv(+_backward), gat_conv(+_backward), mpnn_layer(+_backward)
+    tag_conv(+_backward), gcn_conv(+_backward), gat_conv(+_backward), gat_conv_heads(+_backward), mpnn_layer(+_backward)
 """
 from typing import List, Optional, Tuple
 
@@ -312,6 +312,84 @@ def _gat_backward(ctx, dout, *_unused):
 
 
 gat_conv.register_autograd(_gat_backward, setup_context=_gat_setup)
+
+
+# ----------------------------------------------------------------------------------- GATConv (any heads)
+@_lib.custom_op("dcb200::gat_conv_heads", mutates_args=())
+def gat_conv_heads(x: Tensor, edge_index: Tensor, weight: Tensor, att_src: Tensor, att_dst: Tensor, bias: Optional[Tensor],
+                   negative_slope: float, heads: int, concat: bool, relu: bool, precision: int,
+                   ptr: Optional[List[int]]) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """PyG 2.5.x GATConv(heads=H, concat=...): xs = x W^T viewed as [N, H, C]; per head a_s, a_d, the per-receiver softmax incl.
+    the appended self loop and the weighted sum; out = [N, H*C] (concat) or the mean over heads [N, C], + bias.  Softmax and
+    aggregation are one launch (dc_gat_aggregate).  -> (out, xs, a_src [N, H], a_dst [N, H], alpha_edge [max(E,1), H],
+    alpha_self [N, H]); all but ``out`` are kept for the backward."""
+    g = _csr(edge_index, x.shape[0], "gat", ptr)
+    x = x.contiguous()
+    N, HC = x.shape[0], weight.shape[0]
+    C_ = HC // heads
+    xs = ops.gemm([(x, weight)], N, HC, False, True, precision=precision)
+    a_src, a_dst = ops.gat_scores(xs, att_src.reshape(-1), att_dst.reshape(-1), heads, C_)
+    out, alpha_e, alpha_s = ops.gat_aggregate(g, xs, a_src, a_dst, negative_slope, heads, C_, concat, bias=bias, relu=relu)
+    return out, xs, a_src, a_dst, alpha_e, alpha_s
+
+
+@gat_conv_heads.register_fake
+def _(x, edge_index, weight, att_src, att_dst, bias, negative_slope, heads, concat, relu, precision, ptr):
+    N, HC = x.shape[0], weight.shape[0]
+    return (x.new_empty((N, HC if concat else HC // heads)), x.new_empty((N, HC)), x.new_empty((N, heads)), x.new_empty((N, heads)),
+            x.new_empty((max(edge_index.shape[1], 1), heads)), x.new_empty((N, heads)))
+
+
+@_lib.custom_op("dcb200::gat_conv_heads_backward", mutates_args=())
+def gat_conv_heads_backward(dout: Tensor, out: Tensor, x: Tensor, edge_index: Tensor, weight: Tensor, att_src: Tensor,
+                            att_dst: Tensor, xs: Tensor, a_src: Tensor, a_dst: Tensor, alpha_e: Tensor, alpha_s: Tensor,
+                            negative_slope: float, heads: int, concat: bool, relu: bool, precision: int, ptr: Optional[List[int]],
+                            need_dx: bool, need_db: bool) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
+    """-> (dx, dW, datt_src, datt_dst, dbias); empty tensors for gradients that are not needed.  dz and da_dst by receiver
+    (dc_gat_bwd_edge_heads), then dxs and da_src in one pass by source (dc_gat_scatter_heads), datt by a column reduction."""
+    g = _csr(edge_index, x.shape[0], "gat", ptr)
+    dout, db = ops.relu_bwd_db(out, dout.contiguous(), relu, need_db)
+    N, Fi = x.shape
+    HC = weight.shape[0]
+    C_ = HC // heads
+    x = x.contiguous()
+    db = db if need_db else dout.new_empty(0)
+    dz_e, dz_s, da_dst = ops.gat_bwd_edge_heads(g, a_src, a_dst, negative_slope, alpha_e, alpha_s, xs, dout, heads, C_, concat)
+    dxs, da_src = ops.gat_scatter_heads(g, alpha_e, alpha_s, dz_e, dz_s, da_dst, att_src, att_dst, dout, heads, C_, concat)
+    datt_s, datt_d = ops.gat_att_grad(xs, da_src, da_dst, heads, C_)
+    dx = ops.gemm([(dxs, weight)], N, Fi, False, False, precision=precision) if need_dx else dout.new_empty(0)
+    dw = ops.gemm([(dxs, x)], HC, Fi, True, False, precision=precision)
+    return dx, dw, datt_s.reshape(att_src.shape), datt_d.reshape(att_dst.shape), db
+
+
+@gat_conv_heads_backward.register_fake
+def _(dout, out, x, edge_index, weight, att_src, att_dst, xs, a_src, a_dst, alpha_e, alpha_s, negative_slope, heads, concat, relu,
+      precision, ptr, need_dx, need_db):
+    return (torch.empty_like(x) if need_dx else x.new_empty(0), torch.empty_like(weight), torch.empty_like(att_src),
+            torch.empty_like(att_dst), x.new_empty(dout.shape[1]) if need_db else x.new_empty(0))
+
+
+def _gat_heads_setup(ctx, inputs, output):
+    x, edge_index, weight, att_src, att_dst, bias, slope, heads, concat, relu, precision, ptr = inputs
+    out, xs, a_src, a_dst, alpha_e, alpha_s = output
+    ctx.meta = (slope, heads, concat, relu, precision, ptr, bias is not None)
+    ctx.save_for_backward(out, x, edge_index, weight, att_src, att_dst, xs, a_src, a_dst, alpha_e, alpha_s)
+    ctx.set_materialize_grads(False)
+
+
+def _gat_heads_backward(ctx, dout, *_unused):
+    slope, heads, concat, relu, precision, ptr, has_bias = ctx.meta
+    out, x, edge_index, weight, att_src, att_dst, xs, a_src, a_dst, alpha_e, alpha_s = ctx.saved_tensors
+    if dout is None:
+        return (None,) * 12
+    need_dx, need_db = ctx.needs_input_grad[0], has_bias and ctx.needs_input_grad[5]
+    dx, dw, das, dad, db = torch.ops.dcb200.gat_conv_heads_backward(dout, out, x, edge_index, weight, att_src, att_dst, xs, a_src,
+                                                                    a_dst, alpha_e, alpha_s, slope, heads, concat, relu, precision,
+                                                                    ptr, need_dx, need_db)
+    return (dx if need_dx else None, None, dw, das, dad, db if need_db else None, None, None, None, None, None, None)
+
+
+gat_conv_heads.register_autograd(_gat_heads_backward, setup_context=_gat_heads_setup)
 
 
 # ----------------------------------------------------------------------------------- MPNN layer (A9 extension)

@@ -376,7 +376,7 @@ DC_API int dc_gat_scores(const float* xs, int64_t ld, int64_t num_nodes, int32_t
                   const float* att_dst, float* a_src, float* a_dst, dc_stream_t stream);
 /* Per receiver i over its CSR edges plus the appended self loop:
  *   e = leaky_relu(a_src[nbr] + a_dst[i], slope); alpha = exp(e - max) / (sum + 1e-16).
- * Writes alpha_edge [E] indexed by ORIGINAL edge id (eid[p]) and alpha_self [N]; heads == 1 only. */
+ * Writes alpha_edge [E] indexed by ORIGINAL edge id (eid[p]) and alpha_self [N]; heads == 1 only (any heads: dc_gat_aggregate). */
 DC_API int dc_gat_softmax(const int32_t* rowptr, const int32_t* nbr, const int32_t* eid, const float* a_src,
                    const float* a_dst, float slope, int64_t num_nodes, float* alpha_edge, float* alpha_self,
                    dc_stream_t stream);
@@ -390,6 +390,46 @@ DC_API int dc_gat_bwd_edge(const int32_t* rowptr, const int32_t* nbr, const int3
 /* out[i] = (init ? init[i] : 0) + sum_{p in row i} val[eid[p]]  (CSR order; e.g. da_src over the by-source CSR) */
 DC_API int dc_segment_sum(const int32_t* rowptr, const int32_t* eid, const float* val, const float* init,
                    int64_t num_nodes, float* out, dc_stream_t stream);
+
+/* ---------------------------------------------------------------- K6 multi-head (csrc/gat.cu)
+ * PyG 2.5.x GATConv with any heads >= 1, concat or mean (add_self_loops=True, dropout=0).  Structure: the "gat" CSR pair
+ * (self loops removed; one appended per node by the kernels).  Per-(node, head) arrays are [N, H] row-major, per-edge ones
+ * [E, H] indexed by ORIGINAL edge id.  Sums per (node, head) in CSR order, then the self loop; no atomics.
+ * All return DC_EINVAL for heads < 1, C < 1, a leading dimension shorter than the row, or a null pointer. */
+/* Replaces GATConv's softmax (utils/softmax.py) + propagate(aggr='add') + concat / mean(dim=1) + bias (nn/conv/gat_conv.py):
+ *   z[e,h] = leaky_relu(a_src[src,h] + a_dst[i,h], slope); alpha = exp(z - max_i) / (sum_i exp(z - max_i) + 1e-16);
+ *   out_h[i] = sum_e alpha[e,h] xs[src_e, h*C : (h+1)*C] (+ self loop);
+ *   out[i] = concat ? [out_0 | ... | out_{H-1}] : (out_0 + ... + out_{H-1}) / H;  then + bias (H*C or C), ReLU if relu.
+ * xs [N, H*C] (ld ldx), a_src / a_dst [N, H] from dc_gat_scores.  Writes out (width H*C or C, ld ldo), alpha_edge [E, H],
+ * alpha_self [N, H]. */
+DC_API int dc_gat_aggregate(const int32_t* rowptr, const int32_t* nbr, const int32_t* eid, const float* xs, int64_t ldx,
+                     const float* a_src, const float* a_dst, float slope, int32_t heads, int32_t C, int32_t concat,
+                     const float* bias, int32_t relu, int64_t num_nodes, float* out, int64_t ldo, float* alpha_edge,
+                     float* alpha_self, dc_stream_t stream);
+/* Replaces the autograd of GATConv's attention (softmax and leaky-ReLU backward), by receiver:
+ *   dalpha[e,h] = dout_scale * <dout[i, h*dout_head_stride : +C], xs[src_e, h*C : (h+1)*C]>
+ * (concat: head stride C, scale 1; mean: head stride 0, scale 1/H), then dz = alpha (dalpha - sum alpha dalpha) leaky'(z).
+ * Writes dz_edge [E, H] (by original edge id), dz_self [N, H], da_dst[i,h] = sum of dz over i's edges and self loop. */
+DC_API int dc_gat_bwd_edge_heads(const int32_t* rowptr, const int32_t* nbr, const int32_t* eid, const float* a_src,
+                          const float* a_dst, float slope, const float* alpha_edge, const float* alpha_self, const float* xs,
+                          int64_t ldx, const float* dout, int64_t ldd, int64_t dout_head_stride, float dout_scale,
+                          int32_t heads, int32_t C, int64_t num_nodes, float* dz_edge, float* dz_self, float* da_dst,
+                          dc_stream_t stream);
+/* Replaces the autograd of the aggregation and of the scores (the transposed propagate and the att products), by source, on the
+ * by-source CSR (nbr_t = receivers):  da_src[j,h] = sum_{e: src=j} dz[e,h] + dz_self[j,h];
+ *   dxs[j,h,:] = dout_scale (sum_e alpha[e,h] dout_h[dst_e] + alpha_self[j,h] dout_h[j]) + da_src[j,h] att_src[h,:]
+ *                + da_dst[j,h] att_dst[h,:],  dout_h as in dc_gat_bwd_edge_heads.  Writes dxs [N, H*C] (ld lddx), da_src [N, H]. */
+DC_API int dc_gat_scatter_heads(const int32_t* rowptr_t, const int32_t* nbr_t, const int32_t* eid_t, const float* alpha_edge,
+                         const float* alpha_self, const float* dz_edge, const float* dz_self, const float* da_dst,
+                         const float* att_src, const float* att_dst, const float* dout, int64_t ldd, int64_t dout_head_stride,
+                         float dout_scale, int32_t heads, int32_t C, int64_t num_nodes, float* dxs, int64_t lddx, float* da_src,
+                         dc_stream_t stream);
+/* Replaces the autograd of (xs * att_src).sum(-1) / (xs * att_dst).sum(-1) wrt att:
+ *   datt_src[h,c] = sum_n da_src[n,h] xs[n, h*C + c], datt_dst likewise; fixed two-stage column reduction (as dc_colsum). */
+DC_API size_t dc_gat_att_grad_workspace_bytes(int64_t num_nodes, int32_t heads, int32_t C);
+DC_API int dc_gat_att_grad(const float* xs, int64_t ldx, const float* da_src, const float* da_dst, int64_t num_nodes,
+                    int32_t heads, int32_t C, float* datt_src, float* datt_dst, void* workspace, size_t workspace_bytes,
+                    dc_stream_t stream);
 
 #ifdef __cplusplus
 }
