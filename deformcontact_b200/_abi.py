@@ -32,6 +32,10 @@ class Hop(C.Structure):
                 ("ldout", C.c_int64)]
 
 
+class SddmmPair(C.Structure):
+    _fields_ = [("g", C.c_void_p), ("ldg", C.c_int64), ("h", C.c_void_p), ("ldh", C.c_int64)]
+
+
 MAX_CHAIN = 4
 MAX_SEGS = 4      # dc_gemm: K-segments per call (csrc/gemm.cu); ops.gemm chains larger lists
 
@@ -101,6 +105,10 @@ PROTOTYPES = {
                                     _p]),
     "dc_gat_att_grad_workspace_bytes": (_sz, [_i64, _i32, _i32]),
     "dc_gat_att_grad": (_int, [_p, _i64, _p, _p, _i64, _i32, _i32, _p, _p, _p, _sz, _p]),
+    "dc_gcn_norm_weighted": (_int, [_p, _i64, _i64, _p, _p, _p, _p, _p, _p, _p, _f32, _int, _int, _p, _p, _p, _p, _p, _p, _p, _p,
+                                    _p]),
+    "dc_edge_sddmm": (_int, [_p, _p, _p, C.POINTER(SddmmPair), _i32, _i64, _i32, _int, _p, _p, _p]),
+    "dc_gcn_norm_weighted_backward": (_int, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _i64, _p, _p]),
 }
 
 _lib = None

@@ -282,7 +282,10 @@ class GraphCSR:
     mode "gcn": ``add_remaining_self_loops`` — existing loops dropped, one appended per node.
     mode "gat": ``remove_self_loops`` + ``add_self_loops`` — same structure as "gcn", no dis.
     ``ptr_host`` (python list, ``Batch.ptr``) lets K1 align its tiles with graph boundaries.
+    ``weighted_view`` gives a per-call copy carrying the norms of a per-edge weight (``weighted`` True).
     """
+
+    weighted = False
 
     def __init__(self, edge_index, num_nodes, mode="tag", ptr_host=None, reorder=True):
         if mode not in ("tag", "gcn", "gat", "plain"):
@@ -300,7 +303,7 @@ class GraphCSR:
             rank[self.order.long()] = torch.arange(self.N, dtype=_i64, device=edge_index.device)
             edge_index = rank[edge_index]                      # same edges, same order, new node labels
             self.rank = rank.to(_i32)
-        self.edge_index = edge_index
+        self.edge_index = edge_index.contiguous()     # dense [2, E]: the kernels that read edge_index index it as such
         self.self_loops = mode in ("gcn", "gat")
         self.rowptr, self.nbr, self.eid = csr_build(edge_index, self.N, 0, self.self_loops)
         self.dis = deg_inv_sqrt(self.rowptr, self.N, mode == "gcn") if mode in ("tag", "gcn") else None
@@ -347,6 +350,8 @@ class GraphCSR:
     def t(self):
         """(rowptr, nbr, eid) grouped by source — the transposed structure."""
         if self._t is None:
+            if self.weighted:
+                raise _abi.DcError("weighted view built without its by-source structure (weighted_view(..., transpose=True))")
             self._t = csr_build(self.edge_index, self.N, 1, self.self_loops)
             if self.dis is not None:
                 self._wt = edge_weights(self._t[0], self._t[1], self.dis, self.N, False)[0]
@@ -374,6 +379,8 @@ class GraphCSR:
         w = self._wt if transpose else self.w
         self_loop = self.mode == "gcn"
         variant = K1_VARIANT if K1_VARIANT != "auto" else ("blocks" if transpose else "lean")
+        if variant == "blocks" and self.weighted:
+            variant = "lean"      # edge blocks are a host-planned copy per structure; a weighted view lives for one call
         if variant == "blocks" and self.mode in ("tag", "gcn") and _tiled_ok(h, out, add, bias):
             return spmm_blocks(self.blocks(transpose), rp, self._edges_t if transpose else self.edges,
                                self.self_w if self_loop else None, h, add=add, self_loop=self_loop, bias=bias, relu=relu, out=out)
@@ -383,7 +390,88 @@ class GraphCSR:
         if variant != "generic" and self.mode in ("tag", "gcn") and _tiled_ok(h, out, add, bias):
             return spmm_tiled(rp, nb, w, self.self_w if self_loop else None, h, add=add, self_loop=self_loop, bias=bias,
                               relu=relu, out=out, tile_ptr=self.tile_ptr, n_tiles=self.n_tiles)
+        if self.weighted:
+            return spmm(rp, nb, h, edge_w=w, self_w=self.self_w if self_loop else None, add=add, self_loop=self_loop, bias=bias,
+                        relu=relu, out=out)
         return spmm(rp, nb, h, dis=self.dis, add=add, self_loop=self_loop, bias=bias, relu=relu, out=out)
+
+
+def weighted_view(g, edge_weight, normalize=True, fill_value=1.0, transpose=False):
+    """The structure ``g`` ("tag" or "gcn", as built and cached for ``edge_index``) with the norms of ``edge_weight`` (fp32 [E] in
+    the order of the ``edge_index`` ``g`` was built from): a shallow copy like ``internal_view()`` carrying its own ``dis``,
+    ``w`` / ``edges`` (by target) and, with ``transpose``, ``_wt`` / ``_edges_t`` (by source), plus ``self_w``, ``loop_w`` and
+    ``loop_eid`` for "gcn" (``add_remaining_self_loops(fill_value)``).  PyG's weighted gcn_norm, computed on the device for every
+    call (dc_gcn_norm_weighted); the view is never cached and ``g`` is not modified.  ``normalize=False`` ("tag"): norm_e = w_e.
+    ``propagate`` / ``propagate_chain`` run on the view unchanged, on the packed-record kernels."""
+    if g.mode not in ("tag", "gcn"):
+        raise _abi.DcError(f"weighted_view: needs a 'tag' or 'gcn' structure, got {g.mode!r}")
+    _need(edge_weight, _f32, "edge_weight")
+    if edge_weight.dim() != 1 or edge_weight.shape[0] != g.E:
+        raise _abi.DcError(f"edge_weight: expected [{g.E}] (one weight per edge), got {tuple(edge_weight.shape)}")
+    if edge_weight.device != g.rowptr.device:
+        raise _abi.DcError(f"edge_weight is on {edge_weight.device}, the graph on {g.rowptr.device}")
+    ew = edge_weight.contiguous()
+    rpt, nbt, eidt = g.t if transpose else (None, None, None)
+    N, E, dev = g.N, g.E, ew.device
+    loops = g.mode == "gcn"
+    v = copy.copy(g)
+    v.weighted, v._blocks, v._view, v._t = True, {}, None, g._t if transpose else None
+    v.edge_weight = ew
+    v.dis = torch.empty(N, dtype=_f32, device=dev) if normalize else None
+    v.loop_w = torch.empty(N, dtype=_f32, device=dev) if loops else None
+    v.loop_eid = torch.empty(N, dtype=_i32, device=dev) if loops else None
+    v.self_w = torch.empty(N, dtype=_f32, device=dev) if loops else None
+    v.w = torch.empty(max(E, 1), dtype=_f32, device=dev)
+    v.edges = torch.empty((max(E, 1), 2), dtype=_i32, device=dev)
+    v._wt = torch.empty(max(E, 1), dtype=_f32, device=dev) if transpose else None
+    v._edges_t = torch.empty((max(E, 1), 2), dtype=_i32, device=dev) if transpose else None
+    _abi.call("dc_gcn_norm_weighted", _ptr(g.edge_index), E, N, _ptr(g.rowptr), _ptr(g.nbr), _ptr(g.eid), _ptr(rpt), _ptr(nbt),
+              _ptr(eidt), _ptr(ew), float(fill_value), int(bool(normalize)), int(loops), _ptr(v.dis), _ptr(v.loop_w),
+              _ptr(v.loop_eid), _ptr(v.self_w), _ptr(v.w), _ptr(v.edges), _ptr(v._wt), _ptr(v._edges_t), _stream())
+    return v
+
+
+def edge_sddmm(g, pairs, self_term=False):
+    """s[e] = sum_k <G_k[dst_e], H_k[src_e]> by original edge id over ``g``'s by-target rows (and the self term
+    s_self[i] = sum_k <G_k[i], H_k[i]>) for ``pairs`` = [(G_k, H_k)], all [N, F] in the structure's node order -> (s [E],
+    s_self [N] or None); see dc_edge_sddmm.  More than ``_abi.MAX_CHAIN`` pairs are added in groups, in order."""
+    N, F = pairs[0][0].shape
+    s = torch.empty(max(g.E, 1), dtype=_f32, device=pairs[0][0].device)
+    s_self = torch.empty(N, dtype=_f32, device=s.device) if self_term else None
+    # the ABI wants the neighbour and edge-id arrays even without edges; an edgeless graph has empty ones (null pointers), and
+    # then every row is empty and the stand-in is never read
+    nbr, eid = (g.nbr, g.eid) if g.E else (g.rowptr, g.rowptr)
+    for i0 in range(0, len(pairs), _abi.MAX_CHAIN):
+        grp = pairs[i0:i0 + _abi.MAX_CHAIN]
+        arr = (_abi.SddmmPair * len(grp))()
+        for i, (G, H) in enumerate(grp):
+            _need(G, _f32, "G"), _need(H, _f32, "H")
+            if G.shape != (N, F) or H.shape != (N, F):
+                raise _abi.DcError("edge_sddmm: every pair needs [N, F] operands")
+            arr[i] = _abi.SddmmPair(_ptr(G), _rows(G, "G"), _ptr(H), _rows(H, "H"))
+        e0 = _prof_begin()
+        _abi.call("dc_edge_sddmm", _ptr(g.rowptr), _ptr(nbr), _ptr(eid), arr, len(grp), N, F, int(i0 > 0), _ptr(s),
+                  _ptr(s_self), _stream())
+        _prof_end(e0, op="sddmm", F=F, N=N, E=g.E, bytes=sddmm_bytes(N, g.E, F, len(grp), self_term))
+    return (s if g.E else s.new_empty(0)), s_self
+
+
+def sddmm_bytes(N, E, F, pairs, self_term):
+    """Algorithmic DRAM bytes of one dc_edge_sddmm launch: every G_k and H_k row once, the row pointers, neighbour and edge ids,
+    the outputs."""
+    return 4 * (2 * pairs * N * F + (N + 1) + 2 * E + E + (N if self_term else 0))
+
+
+def gcn_norm_backward(v, s, s_self=None):
+    """dL/dedge_weight [E] (original edge order) from s = dL/dnorm of a weighted view built with ``normalize`` and ``transpose``;
+    see dc_gcn_norm_weighted_backward.  ``s_self``: dL/dself_w of a "gcn" view."""
+    rpt, nbt, eidt = v.t
+    dw = torch.empty(max(v.E, 1), dtype=_f32, device=s.device)
+    loops = s_self is not None
+    _abi.call("dc_gcn_norm_weighted_backward", _ptr(v.rowptr), _ptr(v.nbr), _ptr(v.eid), _ptr(rpt), _ptr(nbt), _ptr(eidt),
+              _ptr(v.edge_weight), _ptr(v.dis), _ptr(v.loop_w if loops else None), _ptr(v.loop_eid if loops else None), _ptr(s),
+              _ptr(s_self), v.N, v.E, _ptr(dw), _stream())
+    return dw if v.E else dw.new_empty(0)
 
 
 def _al16(t):

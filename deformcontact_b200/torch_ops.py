@@ -7,7 +7,8 @@ autograd formula whose backward is again a ``dcb200`` op.  This file holds the O
 four layers' forward / backward; the ``nn.Module``s in ``layers.py`` call these ops and nothing else.
 
     csr_build, propagate, linear, knn_table, radius_table, knn_graph, radius_graph,
-    tag_conv(+_backward), gcn_conv(+_backward), gat_conv(+_backward), gat_conv_heads(+_backward), mpnn_layer(+_backward)
+    tag_conv(+_backward), gcn_conv(+_backward), tag_conv_weighted(+_backward), gcn_conv_weighted(+_backward),
+    gat_conv(+_backward), gat_conv_heads(+_backward), mpnn_layer(+_backward)
 """
 from typing import List, Optional, Tuple
 
@@ -86,7 +87,10 @@ def _(pos, r, ptr, loop, max_num_neighbors):
 def tag_conv(x: Tensor, edge_index: Tensor, weights: List[Tensor], bias: Optional[Tensor], relu: bool, normalize: bool,
              precision: int, ptr: Optional[List[int]]) -> Tuple[Tensor, Tensor]:
     """-> (out [N, Fo], hops [N, K*Fi]) ; hops = [A x | A^2 x | ...] is kept for the backward."""
-    g = _csr(edge_index, x.shape[0], "tag" if normalize else "plain", ptr)
+    return _tag_forward(_csr(edge_index, x.shape[0], "tag" if normalize else "plain", ptr), x, weights, bias, relu, precision)
+
+
+def _tag_forward(g, x, weights, bias, relu, precision):
     x = x.contiguous()
     N, Fi = x.shape
     K = len(weights) - 1
@@ -113,6 +117,13 @@ def tag_conv_backward(dout: Tensor, out: Tensor, x: Tensor, hops: Tensor, edge_i
                       need_dw: bool) -> Tuple[Tensor, Tensor, Tensor]:
     """-> (dx, dbias, dW stacked [K+1, Fo, Fi]); empty tensors for gradients that are not needed."""
     g = _csr(edge_index, x.shape[0], "tag" if normalize else "plain", ptr)
+    dx, db, dws, _, _ = _tag_backward_impl(g, dout, out, x, hops, weights, relu, precision, need_dx, need_db, need_dw)
+    return dx, db, dws
+
+
+def _tag_backward_impl(g, dout, out, x, hops, weights, relu, precision, need_dx, need_db, need_dw, need_chain=False):
+    """-> (dx, dbias, dWs, dhs, hs): dhs[k] = G_k = dL/dH_k (the totals the transposed chain leaves, structure order) for
+    k >= 1 when ``need_chain`` or ``need_dx`` (and k = 0 with ``need_dx``), hs = [x, A x, ...] in structure order."""
     dout, db = ops.relu_bwd_db(out, dout.contiguous(), relu, need_db)   # ReLU backward + bias gradient in one pass
     dout = g.to_internal(dout)      # the saved hops are in the structure's node order
     N, Fo = dout.shape
@@ -126,28 +137,30 @@ def tag_conv_backward(dout: Tensor, out: Tensor, x: Tensor, hops: Tensor, edge_i
     else:
         dws = dout.new_empty(0)
     db = db if need_db else dout.new_empty(0)
-    if need_dx:
+    dhs = None
+    if need_dx or need_chain:
+        lo = 0 if need_dx else 1        # G_0 = dx is only needed for dx
         if ops.K1_CHAIN >= 2 and K > 0:
             # all dH_k = dOut W_k first — ONE batched tensor-core launch over the K + 1 weights where the shapes allow it (same
             # tiles and arithmetic as K + 1 dc_gemm calls, a quarter of the launches / pipeline ramps) — then the transposed hops as
             # one chain, accumulating in place: dH_{k-1} += A_hat^T g_k
+            dhs = [None] * lo
             if (precision != ops.GEMM_FP32 and ops.FORCE_GEMM_PRECISION != ops.GEMM_FP32 and Fi % 4 == 0 and Fo % 4 == 0
                     and float(N) * Fo * Fi >= 1.0e8 and all(w.stride(0) % 4 == 0 and w.data_ptr() % 16 == 0 for w in weights)):
-                dhs = [torch.empty((N, Fi), dtype=dout.dtype, device=dout.device) for _ in range(K + 1)]
-                ops.gemm_batched([(dout, weights[k], dhs[k]) for k in range(K + 1)], trans_a=False, trans_b=False)
+                dhs += [torch.empty((N, Fi), dtype=dout.dtype, device=dout.device) for _ in range(lo, K + 1)]
+                ops.gemm_batched([(dout, weights[k], dhs[k]) for k in range(lo, K + 1)], trans_a=False, trans_b=False)
             else:
-                dhs = [ops.gemm([(dout, weights[k])], N, Fi, False, False, precision=precision) for k in range(K + 1)]
-            ops.propagate_chain(g, [(dhs[k + 1], dhs[k], dhs[k]) for k in range(K - 1, -1, -1)], transpose=True, internal=True)
-            gk = dhs[0]
+                dhs += [ops.gemm([(dout, weights[k])], N, Fi, False, False, precision=precision) for k in range(lo, K + 1)]
+            if K > lo:
+                ops.propagate_chain(g, [(dhs[k + 1], dhs[k], dhs[k]) for k in range(K - 1, lo - 1, -1)], transpose=True, internal=True)
         else:
-            gk = ops.gemm([(dout, weights[K])], N, Fi, False, False, precision=precision)
-            for k in range(K - 1, -1, -1):
+            dhs = [None] * (K + 1)
+            dhs[K] = gk = ops.gemm([(dout, weights[K])], N, Fi, False, False, precision=precision)
+            for k in range(K - 1, lo - 1, -1):
                 dhk = ops.gemm([(dout, weights[k])], N, Fi, False, False, precision=precision)
-                gk = g.propagate(gk, transpose=True, add=dhk, internal=True)
-        dx = g.from_internal(gk)
-    else:
-        dx = dout.new_empty(0)
-    return dx, db, dws
+                dhs[k] = gk = g.propagate(gk, transpose=True, add=dhk, internal=True)
+    dx = g.from_internal(dhs[0]) if need_dx else dout.new_empty(0)
+    return dx, db, dws, dhs, hs
 
 
 @tag_conv_backward.register_fake
@@ -180,6 +193,76 @@ def _tag_backward(ctx, dout, dhops):
 
 
 tag_conv.register_autograd(_tag_backward, setup_context=_tag_setup)
+
+
+# ----------------------------------------------------------------------------------- TAGConv with edge weights
+@_lib.custom_op("dcb200::tag_conv_weighted", mutates_args=())
+def tag_conv_weighted(x: Tensor, edge_index: Tensor, edge_weight: Tensor, weights: List[Tensor], bias: Optional[Tensor], relu: bool,
+                      normalize: bool, precision: int, ptr: Optional[List[int]]) -> Tuple[Tensor, Tensor]:
+    """``tag_conv`` with PyG's ``edge_weight`` [E] (edge_index order): the hops run on the weighted view of the "tag" structure
+    (``ops.weighted_view``: gcn_norm(add_self_loops=False) of the weights, or the raw weights without ``normalize``)."""
+    g = ops.weighted_view(_csr(edge_index, x.shape[0], "tag", ptr), edge_weight, normalize)
+    return _tag_forward(g, x, weights, bias, relu, precision)
+
+
+@tag_conv_weighted.register_fake
+def _(x, edge_index, edge_weight, weights, bias, relu, normalize, precision, ptr):
+    K = len(weights) - 1
+    return x.new_empty((x.shape[0], weights[0].shape[0])), x.new_empty((x.shape[0], max(K, 1) * x.shape[1]))
+
+
+@_lib.custom_op("dcb200::tag_conv_weighted_backward", mutates_args=())
+def tag_conv_weighted_backward(dout: Tensor, out: Tensor, x: Tensor, hops: Tensor, edge_index: Tensor, edge_weight: Tensor,
+                               weights: List[Tensor], relu: bool, normalize: bool, precision: int, ptr: Optional[List[int]],
+                               need_dx: bool, need_db: bool, need_dw: bool, need_dew: bool) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    """-> (dx, dbias, dW stacked, dedge_weight [E]); empty tensors for gradients that are not needed.  dL/dnorm_e =
+    sum_k <G_{k+1}[dst], H_k[src]> in one SDDMM launch over the saved hops and the transposed chain's totals, then the
+    normalisation backward (dc_gcn_norm_weighted_backward)."""
+    g = ops.weighted_view(_csr(edge_index, x.shape[0], "tag", ptr), edge_weight, normalize, transpose=True)
+    dx, db, dws, dhs, hs = _tag_backward_impl(g, dout, out, x, hops, weights, relu, precision, need_dx, need_db, need_dw,
+                                              need_chain=need_dew)
+    K = len(weights) - 1
+    if need_dew and K > 0:
+        s, _ = ops.edge_sddmm(g, [(dhs[k + 1], hs[k]) for k in range(K)])
+        dew = ops.gcn_norm_backward(g, s) if normalize else s
+    elif need_dew:
+        dew = torch.zeros_like(edge_weight)     # K = 0: the output does not depend on the edges
+    else:
+        dew = x.new_empty(0)
+    return dx, db, dws, dew
+
+
+@tag_conv_weighted_backward.register_fake
+def _(dout, out, x, hops, edge_index, edge_weight, weights, relu, normalize, precision, ptr, need_dx, need_db, need_dw, need_dew):
+    return (torch.empty_like(x) if need_dx else x.new_empty(0), x.new_empty(dout.shape[1]) if need_db else x.new_empty(0),
+            x.new_empty((len(weights),) + tuple(weights[0].shape)) if need_dw else x.new_empty(0),
+            torch.empty_like(edge_weight) if need_dew else x.new_empty(0))
+
+
+def _tag_w_setup(ctx, inputs, output):
+    x, edge_index, edge_weight, weights, bias, relu, normalize, precision, ptr = inputs
+    out, hops = output
+    ctx.meta = (relu, normalize, precision, ptr, bias is not None, len(weights))
+    ctx.save_for_backward(out, x, hops, edge_index, edge_weight, *weights)
+    ctx.set_materialize_grads(False)
+
+
+def _tag_w_backward(ctx, dout, dhops):
+    relu, normalize, precision, ptr, has_bias, nw = ctx.meta
+    out, x, hops, edge_index, edge_weight, *weights = ctx.saved_tensors
+    if dout is None:
+        return (None,) * 9
+    need_dx, need_dew = ctx.needs_input_grad[0], ctx.needs_input_grad[2]
+    nig_w = ctx.needs_input_grad[3]
+    need_dw = any(nig_w) if isinstance(nig_w, (list, tuple)) else bool(nig_w)
+    need_db = has_bias and ctx.needs_input_grad[4]
+    dx, db, dws, dew = torch.ops.dcb200.tag_conv_weighted_backward(dout, out, x, hops, edge_index, edge_weight, list(weights), relu,
+                                                                   normalize, precision, ptr, need_dx, need_db, need_dw, need_dew)
+    return (dx if need_dx else None, None, dew if need_dew else None, list(dws.unbind(0)) if need_dw else None,
+            db if need_db else None, None, None, None, None)
+
+
+tag_conv_weighted.register_autograd(_tag_w_backward, setup_context=_tag_w_setup)
 
 
 # ----------------------------------------------------------------------------------- GCNConv
@@ -231,6 +314,72 @@ def _gcn_backward(ctx, dout):
 
 
 gcn_conv.register_autograd(_gcn_backward, setup_context=_gcn_setup)
+
+
+# ----------------------------------------------------------------------------------- GCNConv with edge weights
+@_lib.custom_op("dcb200::gcn_conv_weighted", mutates_args=())
+def gcn_conv_weighted(x: Tensor, edge_index: Tensor, edge_weight: Tensor, weight: Tensor, bias: Optional[Tensor], relu: bool,
+                      fill_value: float, precision: int, ptr: Optional[List[int]]) -> Tuple[Tensor, Tensor]:
+    """``gcn_conv`` with PyG's ``edge_weight`` [E] (edge_index order) and ``add_remaining_self_loops(fill_value)`` (2 for
+    ``improved``): -> (out, xw = x W^T, kept for the backward)."""
+    g = ops.weighted_view(_csr(edge_index, x.shape[0], "gcn", ptr), edge_weight, True, fill_value)
+    xw = ops.gemm([(x.contiguous(), weight)], x.shape[0], weight.shape[0], False, True, precision=precision)
+    return g.propagate(xw, bias=bias, relu=relu), xw
+
+
+@gcn_conv_weighted.register_fake
+def _(x, edge_index, edge_weight, weight, bias, relu, fill_value, precision, ptr):
+    return x.new_empty((x.shape[0], weight.shape[0])), x.new_empty((x.shape[0], weight.shape[0]))
+
+
+@_lib.custom_op("dcb200::gcn_conv_weighted_backward", mutates_args=())
+def gcn_conv_weighted_backward(dout: Tensor, out: Tensor, x: Tensor, xw: Tensor, edge_index: Tensor, edge_weight: Tensor,
+                               weight: Tensor, relu: bool, fill_value: float, precision: int, ptr: Optional[List[int]],
+                               need_dx: bool, need_db: bool, need_dew: bool) -> Tuple[Tensor, Tensor, Tensor, Tensor]:
+    """-> (dx, dW, dbias, dedge_weight [E]); dL/dnorm_e = <dOut[dst], xw[src]> and the loop's <dOut[i], xw[i]> in one SDDMM
+    launch, then the normalisation backward."""
+    g = ops.weighted_view(_csr(edge_index, x.shape[0], "gcn", ptr), edge_weight, True, fill_value, transpose=True)
+    dout, db = ops.relu_bwd_db(out, dout.contiguous(), relu, need_db)
+    N, Fo = dout.shape
+    Fi = x.shape[1]
+    db = db if need_db else dout.new_empty(0)
+    dxw = g.propagate(dout, transpose=True)
+    dx = ops.gemm([(dxw, weight)], N, Fi, False, False, precision=precision) if need_dx else dout.new_empty(0)
+    dw = ops.gemm([(dxw, x.contiguous())], Fo, Fi, True, False, precision=precision)
+    if need_dew:
+        s, s_self = ops.edge_sddmm(g, [(g.to_internal(dout), g.to_internal(xw.contiguous()))], self_term=True)
+        dew = ops.gcn_norm_backward(g, s, s_self)
+    else:
+        dew = dout.new_empty(0)
+    return dx, dw, db, dew
+
+
+@gcn_conv_weighted_backward.register_fake
+def _(dout, out, x, xw, edge_index, edge_weight, weight, relu, fill_value, precision, ptr, need_dx, need_db, need_dew):
+    return (torch.empty_like(x) if need_dx else x.new_empty(0), torch.empty_like(weight),
+            x.new_empty(dout.shape[1]) if need_db else x.new_empty(0), torch.empty_like(edge_weight) if need_dew else x.new_empty(0))
+
+
+def _gcn_w_setup(ctx, inputs, output):
+    x, edge_index, edge_weight, weight, bias, relu, fill_value, precision, ptr = inputs
+    out, xw = output
+    ctx.meta = (relu, fill_value, precision, ptr, bias is not None)
+    ctx.save_for_backward(out, x, xw, edge_index, edge_weight, weight)
+    ctx.set_materialize_grads(False)
+
+
+def _gcn_w_backward(ctx, dout, dxw):
+    relu, fill_value, precision, ptr, has_bias = ctx.meta
+    out, x, xw, edge_index, edge_weight, weight = ctx.saved_tensors
+    if dout is None:
+        return (None,) * 9
+    need_dx, need_dew, need_db = ctx.needs_input_grad[0], ctx.needs_input_grad[2], has_bias and ctx.needs_input_grad[4]
+    dx, dw, db, dew = torch.ops.dcb200.gcn_conv_weighted_backward(dout, out, x, xw, edge_index, edge_weight, weight, relu, fill_value,
+                                                                  precision, ptr, need_dx, need_db, need_dew)
+    return (dx if need_dx else None, None, dew if need_dew else None, dw, db if need_db else None, None, None, None, None)
+
+
+gcn_conv_weighted.register_autograd(_gcn_w_backward, setup_context=_gcn_w_setup)
 
 
 # ----------------------------------------------------------------------------------- GATConv (heads = 1)

@@ -431,6 +431,46 @@ DC_API int dc_gat_att_grad(const float* xs, int64_t ldx, const float* da_src, co
                     int32_t heads, int32_t C, float* datt_src, float* datt_dst, void* workspace, size_t workspace_bytes,
                     dc_stream_t stream);
 
+/* ---------------------------------------------------------------- edge weights for TAGConv / GCNConv (csrc/gcn_norm.cu)
+ * edge_weight: fp32 [E] in edge_index order.  Structures: the "tag" CSR pair (loops kept as ordinary edges) or the "gcn"
+ * pair (self loops dropped, one appended per node).  Per-node sums in CSR order, then the loop; no floating-point atomics. */
+/* Replaces PyG 2.5.2's weighted gcn_norm (nn/conv/gcn_conv.py:gcn_norm; loop_mode 1 = utils/loop.py:add_remaining_self_loops
+ * with fill_value):
+ *   loop_eid[n] = last edge id e with src = dst = n, else -1; loop_w[n] = edge_weight[loop_eid[n]], else fill_value;
+ *   deg_i = sum_{CSR row i} edge_weight[eid] (+ loop_w[i]);  dis = deg^-1/2 (0 where deg == 0, NaN where deg < 0);
+ *   norm_e = (dis[src] * w_e) * dis[dst]  (normalize = 0: norm_e = w_e);  self_w[i] = (dis[i] * loop_w[i]) * dis[i].
+ * Writes dis (normalize), loop_w / loop_eid / self_w (loop_mode 1), and norm_e at every CSR position of the by-target
+ * structure (w_fwd [E] and / or packed {nbr, norm} records edges_fwd [E] for dc_spmm_lean / dc_spmm_chain) and, when
+ * w_src or edges_src is given, of the by-source structure.  edge_index (int64 [2, E]) is read in loop_mode 1 only. */
+DC_API int dc_gcn_norm_weighted(const int64_t* edge_index, int64_t num_edges, int64_t num_nodes, const int32_t* rowptr,
+                                const int32_t* nbr, const int32_t* eid, const int32_t* rowptr_t, const int32_t* nbr_t,
+                                const int32_t* eid_t, const float* edge_weight, float fill_value, int normalize, int loop_mode,
+                                float* dis, float* loop_w, int32_t* loop_eid, float* self_w, float* w_fwd, void* edges_fwd,
+                                float* w_src, void* edges_src, dc_stream_t stream);
+/* Sampled dense-dense products over the edges (the autograd of the hops of MessagePassing.propagate wrt the edge weights):
+ *   s_edge[eid[p]] (+)= sum_k <g_k[i, :F], h_k[nbr[p], :F]>  for every by-target CSR position p of receiver i,
+ *   s_self[i]      (+)= sum_k <g_k[i, :F], h_k[i, :F]>        (when s_self is not NULL),
+ * for 1..DC_MAX_CHAIN pairs in one launch (accumulate = 1 adds to the values already there).  One warp per receiver; per pair
+ * a lane sums its columns in fp32, the pairs and the lanes are added in fp64 (fixed shuffle tree), rounded once.
+ * DC_EINVAL for F < 1, a bad pair count, ld < F or a null pointer (rowptr, nbr, eid, pairs, s_edge and every g_k / h_k are
+ * required; nbr and eid are not read when every row is empty). */
+typedef struct dc_sddmm_pair {
+  const float* g; int64_t ldg;
+  const float* h; int64_t ldh;
+} dc_sddmm_pair_t;
+DC_API int dc_edge_sddmm(const int32_t* rowptr, const int32_t* nbr, const int32_t* eid, const dc_sddmm_pair_t* pairs,
+                         int32_t num_pairs, int64_t num_nodes, int32_t F, int accumulate, float* s_edge, float* s_self,
+                         dc_stream_t stream);
+/* Backward of dc_gcn_norm_weighted (normalize = 1) from s = dL/dnorm (dc_edge_sddmm), in fp64, rounded once:
+ *   dL/ddis_n = sum_{e: dst=n} s_e dis[src] w_e + sum_{e: src=n} s_e w_e dis[dst] + 2 s_self[n] loop_w[n] dis[n];
+ *   dL/ddeg_n = -dis_n^3 / 2 * dL/ddis_n (0 where deg_n == 0);  dw[e] = s_e dis[src] dis[dst] + dL/ddeg[dst];
+ *   dw[loop_eid[n]] = s_self[n] dis[n]^2 + dL/ddeg_n; every other edge (superseded loops, dropped edges) gets 0.
+ * s_self / loop_w / loop_eid NULL: no appended loops (the "tag" structure).  dw [E] by original edge id. */
+DC_API int dc_gcn_norm_weighted_backward(const int32_t* rowptr, const int32_t* nbr, const int32_t* eid, const int32_t* rowptr_t,
+                                         const int32_t* nbr_t, const int32_t* eid_t, const float* edge_weight, const float* dis,
+                                         const float* loop_w, const int32_t* loop_eid, const float* s_edge, const float* s_self,
+                                         int64_t num_nodes, int64_t num_edges, float* dw, dc_stream_t stream);
+
 #ifdef __cplusplus
 }
 #endif
