@@ -24,6 +24,10 @@ extern "C" int dc_gemm_batched(const dc_gemm_problem* problems, int32_t count, i
                                dc_stream_t stream_) {
   DC_REQUIRE(count >= 0, DC_EINVAL, "gemm_batched: negative count");
   if (count == 0) return DC_OK;
+  DC_REQUIRE(problems, DC_EINVAL, "gemm_batched: no problems");
+  for (int32_t i = 0; i < count; ++i)
+    DC_REQUIRE(!(problems[i].E && (relu || accumulate)), DC_EINVAL,
+               "gemm_batched: problem %d: the fused epilogue operand E excludes relu and accumulate", i);
   return dcb::gemm_tc2_batched(problems, count, transA, transB, relu, accumulate, workspace, workspace_bytes, host_staging,
                                host_staging_bytes, (cudaStream_t)stream_);
 }

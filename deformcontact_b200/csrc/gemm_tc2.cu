@@ -21,7 +21,7 @@
 //   * Work item = (row tile, column chunk, k part): when M x N alone gives fewer tiles than SMs the contraction
 //     is cut into parts whose partial tiles go to slabs that a second kernel sums in fixed order (deterministic).
 //   * Template PAIR (round 2): clusters of two CTAs drive one cta_group::2 MMA (M = 256), each CTA loading / splitting half of B.
-//   * Template TEPI (round 2, CTA pairs, K <= 512): TMA epilogue — three stages and a 64 KB epilogue area of per-warp SWIZZLE_128B
+//   * Template TEPI (round 2, CTA pairs; which products take it: t2_tepi_mode): TMA epilogue — three stages and a 64 KB epilogue area of per-warp SWIZZLE_128B
 //     blocks; the fused epilogue operand arrives by TMA while the tile's MMAs run, the output tile leaves by TMA stores
 //     (profiles/r02c_tepi_ab.txt: fused softmax-backward product 12.9 -> 10.0 ms).
 #include <cuda.h>
@@ -863,7 +863,7 @@ int t2_pair() {
 }
 
 // TMA epilogue (CTA pairs only): DCB200_T2_TEPI = 0 off, 1 for short contractions (K <= 512: the products whose tile time is set by
-// the epilogue — attention scores, the fused softmax-backward product, the K = 256 layer products), 2 for every K, 3 (default) = as 1,
+// the epilogue — attention scores, the fused softmax-backward product, the K = 256 layer products), 2 for every K, 3 (default) = as 2,
 // but a batched launch takes it only when a problem carries a fused epilogue operand: the plain batched scores product prefers the
 // fourth pipeline stage (same-box A/B, profiles/r02c_tepi_ab.txt: 92.10 -> 91.79 ms per step)
 int t2_tepi_mode() {
@@ -878,7 +878,12 @@ bool t2_tepi_ok(int pair, int64_t kb_max, int k_parts, int accumulate) {
   const int mode = t2_tepi_mode();
   return pair && mode > 0 && k_parts == 1 && !accumulate && (mode > 1 || kb_max <= T2_SHORT_KB);
 }
-bool t2_tepi_operand_ok(const float* ptr, int64_t ld) { return ptr && (ld & 3) == 0 && (reinterpret_cast<uintptr_t>(ptr) & 15) == 0; }
+// An [M, N] operand the TMA epilogue can address.  N % 4 == 0 as well: the TMA stores of the swizzled output boxes write the whole
+// 16-byte chunk that holds column N - 1, so a row of N % 4 != 0 floats would get up to three floats past its end overwritten
+// (measured on the B200 with C a view into a wider buffer).
+bool t2_tepi_operand_ok(const float* ptr, int64_t ld, int64_t N) {
+  return ptr && (ld & 3) == 0 && (N & 3) == 0 && (reinterpret_cast<uintptr_t>(ptr) & 15) == 0;
+}
 
 // one persistent CTA per SM; PAIR: clusters of two CTAs (an even grid)
 int t2_launch(const CUtensorMap* mA, const CUtensorMap* mB, const CUtensorMap& mC, const T2Params& p, cudaStream_t st) {
@@ -947,7 +952,7 @@ int gemm_tc2(const dc_gemm_seg* segs, int nseg, int transA, int transB, int64_t 
   p.pair = t2_pair();
   const uint32_t b_box_rows = p.pair ? T2_BN / 2 : T2_BN;   // a CTA of a pair loads half of the B tile
   CUtensorMap mA[4], mB[4];
-  int64_t ktot = 0;
+  int64_t ktot = 0, kelems = 0;
   for (int s = 0; s < 4; ++s) {
     const int ss = s < nseg ? s : 0;
     const uint64_t K = (uint64_t)segs[ss].K;
@@ -962,13 +967,15 @@ int gemm_tc2(const dc_gemm_seg* segs, int nseg, int transA, int transB, int64_t 
       if (int rc = make_map2(&mB[s], segs[ss].B, (uint64_t)N, K, (uint64_t)segs[ss].ldb, 32, CU_TENSOR_MAP_SWIZZLE_128B_ATOM_32B)) return rc;
     }
     p.kb_seg[s] = s < nseg ? (int)cdiv(segs[s].K, T2_BK) : (1 << 30);
-    if (s < nseg) ktot += cdiv(segs[s].K, T2_BK);
+    if (s < nseg) ktot += cdiv(segs[s].K, T2_BK), kelems += segs[s].K;
   }
   p.kb_total = (int)ktot;
   p.M = (int)M; p.N = (int)N;
   p.m_tiles = (int)cdiv(M, T2_BM);
   p.n_chunks = (int)cdiv(N, T2_BN);
-  p.k_parts = t2_k_parts(M, N, p.kb_total);
+  // the number of parts follows the contraction length, as in gemm_tc2_workspace_bytes: segments whose K is not a multiple of
+  // 32 each add a partial k-block, which must not raise the part count above what the workspace query promised
+  p.k_parts = t2_k_parts(M, N, cdiv(kelems, T2_BK));
   p.kb_per_part = (int)(cdiv(cdiv(p.kb_total, p.k_parts), T2_PART_KB) * T2_PART_KB);   // whole chains per part
   p.k_parts = (int)cdiv(p.kb_total, p.kb_per_part);
   p.items = (p.pair ? (p.m_tiles + 1) / 2 : p.m_tiles) * p.n_chunks * p.k_parts;   // pair: items are pairs of row tiles
@@ -985,7 +992,7 @@ int gemm_tc2(const dc_gemm_seg* segs, int nseg, int transA, int transB, int64_t 
     p.partial = reinterpret_cast<float*>((reinterpret_cast<uintptr_t>(workspace) + 255) & ~(uintptr_t)255);
   }
   CUtensorMap mC{};
-  p.tepi = t2_tepi_ok(p.pair, p.kb_total, p.k_parts, accumulate) && t2_tepi_operand_ok(C, ldc);
+  p.tepi = t2_tepi_ok(p.pair, p.kb_total, p.k_parts, accumulate) && t2_tepi_operand_ok(C, ldc, N);
   if (p.tepi)
     if (int rc = make_map2(&mC, C, (uint64_t)N, (uint64_t)M, (uint64_t)ldc, 32, CU_TENSOR_MAP_SWIZZLE_128B)) return rc;
   if (int rc = t2_launch(mA, mB, mC, p, st)) return rc;
@@ -1038,7 +1045,7 @@ int gemm_tc2_batched(const dc_gemm_problem* probs, int count, int transA, int tr
     const dc_gemm_problem& q = probs[i];
     if (q.M <= 0 || q.N <= 0) continue;
     if (cdiv(q.K, T2_BK) > kb_all) kb_all = cdiv(q.K, T2_BK);
-    if (!t2_tepi_operand_ok(q.C, q.ldc) || (q.E && !t2_tepi_operand_ok(q.E, q.lde))) tepi_operands = false;
+    if (!t2_tepi_operand_ok(q.C, q.ldc, q.N) || (q.E && !t2_tepi_operand_ok(q.E, q.lde, q.N))) tepi_operands = false;
   }
   // mode 3 (lab): batched launches take the TMA epilogue only when a problem carries a fused epilogue operand
   bool any_e = false;

@@ -794,7 +794,10 @@ def gemm(segs, M, N, trans_a=False, trans_b=True, bias=None, relu=False, out=Non
 def gemm_batched(problems, trans_a=False, trans_b=True, relu=False, accumulate=False):
     """problems = [(A, B, C), ...]: C_i = act(opA(A_i) opB(B_i)) (+C_i) for all i in one tensor-core launch; see
     dc_gemm_batched.  A problem may carry a fused epilogue (A, B, C, E, rowv): C = E o (acc - rowv[:, None]).
-    Falls back to one dc_gemm per problem when a problem does not fit the tensor path."""
+    Falls back to one dc_gemm per problem when a problem does not fit the tensor path.  The fused epilogue excludes
+    ``relu`` and ``accumulate``, as in dc_gemm_batched."""
+    if (relu or accumulate) and any(len(q) > 3 for q in problems):
+        raise _abi.DcError("gemm_batched: the fused epilogue operand E excludes relu and accumulate")
     problems = [q for q in problems if q[2].numel() > 0]
     if not problems:
         return

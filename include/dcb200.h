@@ -241,7 +241,7 @@ typedef struct {
   const float* E;    /* optional fused epilogue: C = E o (acc - rowv[row]) with E [M, N] (lde), rowv [M]; NULL = none. */
   int64_t lde;       /* With E = P (attention weights) and rowv = rowdot(dO, O) this is the softmax backward          */
   const float* rowv; /* dS = P o (dP - rowsum(dP o P)) applied to dP = dO Xr^T as it leaves the tensor core.          */
-} dc_gemm_problem;
+} dc_gemm_problem;   /* A batch in which any problem carries E must have relu = 0 and accumulate = 0 (DC_EINVAL otherwise). */
 DC_API size_t dc_gemm_batched_workspace_bytes(int32_t count);
 DC_API int dc_gemm_batched(const dc_gemm_problem* problems /*host array*/, int32_t count, int transA, int transB, int relu,
                            int accumulate, void* workspace, size_t workspace_bytes, void* host_staging /*pinned host or NULL*/,

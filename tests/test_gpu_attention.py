@@ -248,3 +248,45 @@ def test_gemm_tma_epilogue_equals_the_staged_epilogue_bit_for_bit(dc):
             assert torch.equal(out_tma, out_staged), (M, N, K, relu)
             ref = A.double() @ B.double().T + b.double()
             assert_close(out_tma, (ref.relu() if relu else ref).float(), what="TMA epilogue bias / relu")
+
+
+@pytest.mark.parametrize("case", ["three_heads", "empty_groups", "peaked"])
+def test_cross_attention_heads_empty_groups_peaked(dc, case):
+    """_AttnFn over H = 3 heads (one batched launch per product type over heads x groups; dxs and dxr summed over heads),
+    a group without resting nodes next to a group without collider nodes (the zero fills of rows no live group writes), and
+    a peaked softmax (row max P >= 0.9 on most rows), where the unscaled softmax amplifies score error."""
+    from deformcontact_b200 import attention
+    H, ptr_s, ptr_r, wscale = {
+        "three_heads": (3, [0, 300, 700, 1000], [0, 40, 100, 180], 0.5),
+        "empty_groups": (2, [0, 300, 300, 700, 1000], [0, 40, 90, 90, 150], 0.5),
+        "peaked": (1, [0, 500, 1000], [0, 200, 400], 6.0),
+    }[case]
+    F = 64
+    g = torch.Generator().manual_seed(11)
+    Ns, Nr = ptr_s[-1], ptr_r[-1]
+    xs = torch.randn(Ns, F, generator=g).relu()
+    xr = torch.randn(Nr, F, generator=g).relu()
+    params = []
+    for _ in range(H):
+        params += [(torch.rand(F, F, generator=g) * 2 - 1) / F ** 0.5 * wscale, (torch.rand(F, generator=g) * 2 - 1) / F ** 0.5]
+    gos = [torch.randn(Ns, F, generator=g) for _ in range(H)]
+    groups = attention._groups(ptr_s, ptr_r, 1)
+    if case == "peaked":
+        W, b = params
+        pmax = torch.cat([torch.softmax((xs[s0:s1] @ W.T + b) @ (xr[r0:r1] @ W.T + b).T, -1).max(-1).values
+                          for s0, s1, r0, r1 in groups])
+        assert (pmax >= 0.9).float().mean() >= 0.8
+
+    def run(dtype, dev):
+        t = [v.detach().clone().to(dtype=dtype, device=dev).requires_grad_(True) for v in [xs, xr] + params]
+        if dev == "cuda":
+            outs = attention._AttnFn.apply(t[0], t[1], groups, *t[2:])
+        else:
+            outs = [_ref(t[0], t[1], t[2 + 2 * h], t[3 + 2 * h], groups) for h in range(H)]
+        sum((o * go.to(dtype=dtype, device=dev)).sum() for o, go in zip(outs, gos)).backward()
+        return list(outs) + [v.grad for v in t]
+
+    ours, r32, r64 = run(torch.float32, "cuda"), run(torch.float32, "cpu"), run(torch.float64, "cpu")
+    names = [f"out{h}" for h in range(H)] + ["dxs", "dxr"] + [f"{n}{h}" for h in range(H) for n in ("dW", "db")]
+    for name, a, b32, b64 in zip(names, ours, r32, r64):
+        assert_close_arbiter(a, b32, b64, what=f"attention {case} {name}")
