@@ -101,6 +101,8 @@ PROTOTYPES = {
     "dc_gat_aggregate": (_int, [_p, _p, _p, _p, _i64, _p, _p, _f32, _i32, _i32, _i32, _p, _i32, _i64, _p, _i64, _p, _p, _p]),
     "dc_gat_bwd_edge_heads": (_int, [_p, _p, _p, _p, _p, _f32, _p, _p, _p, _i64, _p, _i64, _i64, _f32, _i32, _i32, _i64, _p, _p, _p,
                                      _p]),
+    "dc_gat_bwd_edge_heads_ext": (_int, [_p, _p, _p, _p, _p, _f32, _p, _p, _p, _i64, _p, _i64, _i64, _f32, _i32, _i32, _i64, _p, _p,
+                                         _p, _p, _p, _p]),
     "dc_gat_scatter_heads": (_int, [_p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _p, _i64, _i64, _f32, _i32, _i32, _i64, _p, _i64, _p,
                                     _p]),
     "dc_gat_att_grad_workspace_bytes": (_sz, [_i64, _i32, _i32]),

@@ -114,17 +114,19 @@ gat_aggregate_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restri
 }
 
 // Backward by receiver.  Phase 1: i's (edge, head) pairs — CSR edges, then the self loop — are spread over the lanes; a lane takes
-// dalpha = scale * <dout[i, h*hs : h*hs + C], xs[j, h*C : (h+1)*C]> sequentially (fp64 accumulator, for the same reason)
+// dalpha = scale * <dout[i, h*hs : h*hs + C], xs[j, h*C : (h+1)*C]> sequentially (fp64 accumulator, for the same reason),
+// with EXT adds the gradient that reaches alpha itself (dalpha_edge [E, H] by edge id, dalpha_self [N, H]; either may be null),
 // and stashes it in dz_edge / dz_self.  Phase 2
 // (lane = head): s = sum alpha * dalpha in CSR order then the self loop; dz = alpha * (dalpha - s) * leaky_relu'(z), written over
 // the stash; da_dst[i, h] = sum of dz in the same order.
-template <int VEC, int G>
+template <int VEC, int G, bool EXT>
 __global__ void __launch_bounds__(256)
 gat_bwd_edge_heads_kernel(const int32_t* __restrict__ rowptr, const int32_t* __restrict__ nbr, const int32_t* __restrict__ eid,
                           const float* __restrict__ a_src, const float* __restrict__ a_dst, float slope,
                           const float* __restrict__ alpha_edge, const float* __restrict__ alpha_self, const float* __restrict__ xs,
                           int64_t ldx, const float* __restrict__ dout, int64_t ldd, int64_t hs, float scale, int H, int C, int64_t N,
-                          float* dz_edge, float* dz_self, float* __restrict__ da_dst) {
+                          const float* __restrict__ dalpha_edge, const float* __restrict__ dalpha_self, float* dz_edge,
+                          float* dz_self, float* __restrict__ da_dst) {
   const int l = threadIdx.x % G;
   const int64_t i = (int64_t)blockIdx.x * (256 / G) + threadIdx.x / G;
   const bool live = i < N;
@@ -145,9 +147,14 @@ gat_bwd_edge_heads_kernel(const int32_t* __restrict__ rowptr, const int32_t* __r
 #pragma unroll
         for (int u = 0; u < VEC; ++u) acc = fma((double)y.v[u], (double)x.v[u], acc);
       }
-      const float d = __fmul_rn((float)acc, scale);
-      if (self) dz_self[i * H + h] = d;
-      else dz_edge[(int64_t)eid[p] * H + h] = d;
+      float d = __fmul_rn((float)acc, scale);
+      const int64_t k = self ? i * H + h : (int64_t)eid[p] * H + h;
+      if constexpr (EXT) {
+        const float* ext = self ? dalpha_self : dalpha_edge;
+        if (ext) d = __fadd_rn(d, ext[k]);
+      }
+      if (self) dz_self[k] = d;
+      else dz_edge[k] = d;
     }
   }
   __syncwarp();
@@ -303,11 +310,14 @@ extern "C" int dc_gat_aggregate(const int32_t* rowptr, const int32_t* nbr, const
   return DC_OK;
 }
 
-extern "C" int dc_gat_bwd_edge_heads(const int32_t* rowptr, const int32_t* nbr, const int32_t* eid, const float* a_src,
-                                     const float* a_dst, float slope, const float* alpha_edge, const float* alpha_self, const float* xs,
-                                     int64_t ldx, const float* dout, int64_t ldd, int64_t dout_head_stride, float dout_scale, int32_t H,
-                                     int32_t C, int64_t N, float* dz_edge, float* dz_self, float* da_dst, dc_stream_t stream_) {
-  cudaStream_t st = (cudaStream_t)stream_;
+namespace {
+// Both by-receiver entry points: the same checks, then the kernel without (EXT false) or with the external alpha gradient.
+template <bool EXT>
+int gat_bwd_edge_heads_launch(const int32_t* rowptr, const int32_t* nbr, const int32_t* eid, const float* a_src, const float* a_dst,
+                              float slope, const float* alpha_edge, const float* alpha_self, const float* xs, int64_t ldx,
+                              const float* dout, int64_t ldd, int64_t dout_head_stride, float dout_scale, int32_t H, int32_t C,
+                              int64_t N, const float* dalpha_edge, const float* dalpha_self, float* dz_edge, float* dz_self,
+                              float* da_dst, cudaStream_t st) {
   DC_REQUIRE(H >= 1 && C >= 1 && N >= 0 && dout_head_stride >= 0, DC_EINVAL, "gat_bwd_edge_heads: heads and C must be >= 1");
   DC_REQUIRE(ldx >= (int64_t)H * C && ldd >= (int64_t)(H - 1) * dout_head_stride + C, DC_EINVAL,
              "gat_bwd_edge_heads: ld smaller than the row");
@@ -316,14 +326,39 @@ extern "C" int dc_gat_bwd_edge_heads(const int32_t* rowptr, const int32_t* nbr, 
              DC_EINVAL, "gat_bwd_edge_heads: null pointer");
   const int vec = (C % 4 == 0 && ldx % 4 == 0 && ldd % 4 == 0 && dout_head_stride % 4 == 0 && al16(xs) && al16(dout)) ? 4 : 1;
   const int G = group_width(9 * (int64_t)H);     // pairs of a receiver of degree 8
-#define DC_GAT_BWD(V, GG)                                                                                                       \
-  gat_bwd_edge_heads_kernel<V, GG><<<(unsigned)cdiv(N, 256 / GG), 256, 0, st>>>(rowptr, nbr, eid, a_src, a_dst, slope, alpha_edge,  \
-                                                                              alpha_self, xs, ldx, dout, ldd, dout_head_stride,  \
-                                                                              dout_scale, H, C, N, dz_edge, dz_self, da_dst)
+#define DC_GAT_BWD(V, GG)                                                                                                        \
+  gat_bwd_edge_heads_kernel<V, GG, EXT><<<(unsigned)cdiv(N, 256 / GG), 256, 0, st>>>(                                            \
+      rowptr, nbr, eid, a_src, a_dst, slope, alpha_edge, alpha_self, xs, ldx, dout, ldd, dout_head_stride, dout_scale, H, C, N,  \
+      dalpha_edge, dalpha_self, dz_edge, dz_self, da_dst)
   DC_GAT_DISPATCH(vec, G, DC_GAT_BWD);
 #undef DC_GAT_BWD
   DC_LAUNCH_CHECK();
   return DC_OK;
+}
+}  // namespace
+
+extern "C" int dc_gat_bwd_edge_heads(const int32_t* rowptr, const int32_t* nbr, const int32_t* eid, const float* a_src,
+                                     const float* a_dst, float slope, const float* alpha_edge, const float* alpha_self, const float* xs,
+                                     int64_t ldx, const float* dout, int64_t ldd, int64_t dout_head_stride, float dout_scale, int32_t H,
+                                     int32_t C, int64_t N, float* dz_edge, float* dz_self, float* da_dst, dc_stream_t stream_) {
+  return gat_bwd_edge_heads_launch<false>(rowptr, nbr, eid, a_src, a_dst, slope, alpha_edge, alpha_self, xs, ldx, dout, ldd,
+                                          dout_head_stride, dout_scale, H, C, N, nullptr, nullptr, dz_edge, dz_self, da_dst,
+                                          (cudaStream_t)stream_);
+}
+
+extern "C" int dc_gat_bwd_edge_heads_ext(const int32_t* rowptr, const int32_t* nbr, const int32_t* eid, const float* a_src,
+                                         const float* a_dst, float slope, const float* alpha_edge, const float* alpha_self,
+                                         const float* xs, int64_t ldx, const float* dout, int64_t ldd, int64_t dout_head_stride,
+                                         float dout_scale, int32_t H, int32_t C, int64_t N, const float* dalpha_edge,
+                                         const float* dalpha_self, float* dz_edge, float* dz_self, float* da_dst,
+                                         dc_stream_t stream_) {
+  if (!dalpha_edge && !dalpha_self)     // nothing to add: the kernel of dc_gat_bwd_edge_heads, bit for bit
+    return gat_bwd_edge_heads_launch<false>(rowptr, nbr, eid, a_src, a_dst, slope, alpha_edge, alpha_self, xs, ldx, dout, ldd,
+                                            dout_head_stride, dout_scale, H, C, N, nullptr, nullptr, dz_edge, dz_self, da_dst,
+                                            (cudaStream_t)stream_);
+  return gat_bwd_edge_heads_launch<true>(rowptr, nbr, eid, a_src, a_dst, slope, alpha_edge, alpha_self, xs, ldx, dout, ldd,
+                                         dout_head_stride, dout_scale, H, C, N, dalpha_edge, dalpha_self, dz_edge, dz_self, da_dst,
+                                         (cudaStream_t)stream_);
 }
 
 extern "C" int dc_gat_scatter_heads(const int32_t* rowptr_t, const int32_t* nbr_t, const int32_t* eid_t, const float* alpha_edge,

@@ -186,7 +186,22 @@ class GATConv(nn.Module):
     ``torch.ops.dcb200.gat_conv_heads``: per-head softmax and aggregation in one launch with the concat / mean epilogue
     (``dc_gat_aggregate``), backward by receiver then by source (``dc_gat_bwd_edge_heads``, ``dc_gat_scatter_heads``).
     Attention dropout, ``add_self_loops=False``, ``fill_value`` and ``edge_dim`` are not supported and raise; the call takes no
-    ``edge_attr``."""
+    ``edge_attr``.
+
+    ``layer(x, edge_index, return_attention_weights=...)`` as in PyG 2.5.2:
+
+    - ``None`` (the default): the output tensor.
+    - any ``bool``, ``False`` included (PyG tests ``isinstance(..., bool)``): ``(out, (edge_index_sl, alpha))``.
+      ``edge_index_sl`` int64 ``[2, E_nl + N]`` is ``add_self_loops(remove_self_loops(edge_index), N)``: the edges that are not
+      self loops in their order (duplicates kept), then one loop per node, in the node labels of ``edge_index`` (of the tensor a
+      prebuilt ``GraphCSR`` was built from).  It is built once per structure and shared by later calls: do not write to it.
+      ``alpha`` fp32 ``[E_nl + N, H]`` (the head axis kept for H = 1) holds the coefficients the aggregation used, row for row,
+      and is differentiable: a loss on ``alpha`` (an entropy or sparsity regulariser) reaches ``x`` and every parameter.
+      ``relu`` applies to ``out`` only.  Any other value raises ``TypeError``.
+
+    With attention weights every ``heads`` runs ``gat_conv_heads``, which keeps alpha per head; the gradient that reaches alpha
+    enters its receiver pass (``dc_gat_bwd_edge_heads_ext``).  For H = 1 ``out`` is therefore within rounding of, not
+    bit-identical to, the call without.  The first call on a structure reads the edge count back to the host once."""
 
     def __init__(self, in_channels, out_channels, heads=1, concat=True, negative_slope=0.2, bias=True, precision=ops.GEMM_AUTO, *,
                  dropout=0.0, add_self_loops=True, edge_dim=None, fill_value="mean"):
@@ -205,13 +220,21 @@ class GATConv(nn.Module):
         self.bias = nn.Parameter(torch.zeros(heads * out_channels if concat else out_channels)) if bias else None
         self.precision = precision
 
-    def forward(self, x, edge_index, relu=False, ptr=None):
-        if self.heads == 1:     # the mean over one head is that head: concat and mean are the same layer
-            return torch.ops.dcb200.gat_conv(x, _edge_tensor(edge_index), self.lin.weight, self.att_src, self.att_dst, self.bias,
+    def forward(self, x, edge_index, relu=False, ptr=None, *, return_attention_weights=None):
+        if return_attention_weights is not None and not isinstance(return_attention_weights, bool):
+            raise TypeError("return_attention_weights must be None or a bool, got "
+                            f"{type(return_attention_weights).__name__}")
+        ei = _edge_tensor(edge_index)
+        if return_attention_weights is None and self.heads == 1:   # the mean over one head is that head: concat = mean
+            return torch.ops.dcb200.gat_conv(x, ei, self.lin.weight, self.att_src, self.att_dst, self.bias,
                                              float(self.negative_slope), relu, self.precision, ptr)[0]
-        return torch.ops.dcb200.gat_conv_heads(x, _edge_tensor(edge_index), self.lin.weight, self.att_src, self.att_dst, self.bias,
-                                               float(self.negative_slope), self.heads, bool(self.concat), relu, self.precision,
-                                               ptr)[0]
+        res = torch.ops.dcb200.gat_conv_heads(x, ei, self.lin.weight, self.att_src, self.att_dst, self.bias,
+                                              float(self.negative_slope), self.heads, bool(self.concat), relu, self.precision, ptr)
+        if return_attention_weights is None:
+            return res[0]
+        g = ops.graph_csr(ei, x.shape[0], "gat", list(ptr) if ptr is not None else None)
+        keep, edge_index_sl = g.attention_edges()
+        return res[0], (edge_index_sl, ops.attention_weights(res[4], res[5], keep, g.E))
 
 
 # ------------------------------------------------------------------------------- MPNN (A9 extension)

@@ -323,6 +323,7 @@ class GraphCSR:
         self._blocks = {}
         self._max_tile = max((b - a for a, b in zip(tiles[:-1], tiles[1:])), default=0) if tiles is not None else TILE_NODES
         self._view = None
+        self._att = None
 
     def internal_view(self):
         """The same structure seen as a graph whose nodes ARE numbered in this structure's order (``order`` None).  A stack of
@@ -345,6 +346,22 @@ class GraphCSR:
             rp = self.t[0] if transpose else self.rowptr
             self._blocks[key] = EdgeBlocks(rp, self._edges_t if transpose else self.edges, self.N, self.E, self._tiles_host, unit)
         return self._blocks[key]
+
+    def attention_edges(self):
+        """(keep, edge_index_sl) of a "gat" structure, built on first use and kept: ``keep`` int64 [E_nl], the ids of the edges
+        that are not self loops, in edge order, or None when no edge is one (then alpha's edge rows are alpha_e[:E] as they
+        stand, a copy instead of a gather); ``edge_index_sl`` int64 [2, E_nl + N] = ``add_self_loops(remove_self_loops(
+        edge_index), N)``, PyG GATConv's attention edges, in the labels of the tensor the structure was built from.  The first
+        call reads E_nl back to the host (one synchronisation); later calls launch nothing, so they can be captured."""
+        if self.mode != "gat":
+            raise _abi.DcError(f"attention_edges: needs a 'gat' structure, got {self.mode!r}")
+        if self._att is None:
+            ei = self._src_edge_index.to(_i64)
+            keep = torch.nonzero(ei[0] != ei[1]).squeeze(1)
+            loops = torch.arange(self.N, dtype=_i64, device=ei.device)
+            edges = ei[:, keep] if keep.shape[0] < self.E else ei
+            self._att = (keep if keep.shape[0] < self.E else None, torch.cat([edges, loops.expand(2, -1)], 1))
+        return self._att
 
     @property
     def t(self):
@@ -559,6 +576,33 @@ class _PermuteRows(torch.autograd.Function):
     @staticmethod
     def backward(ctx, dout):
         return permute_rows(dout.contiguous(), ctx.inverse), None, None
+
+
+class _AttentionWeights(torch.autograd.Function):
+    """alpha in the order of ``edge_index_sl``: cat(alpha_e[keep], alpha_s) [E_nl + N, H].  The backward writes the gradient
+    back to [max(E, 1), H] by edge id (zeros at self-loop edges; ``keep`` holds each id once, so a plain index copy) and [N, H]."""
+
+    @staticmethod
+    def forward(ctx, alpha_e, alpha_s, keep, E):
+        ctx.keep, ctx.rows, ctx.E = keep, alpha_e.shape[0], E
+        return torch.cat([alpha_e[:E] if keep is None else alpha_e.index_select(0, keep), alpha_s], 0)
+
+    @staticmethod
+    def backward(ctx, dalpha):
+        keep, E = ctx.keep, ctx.E
+        n_keep = E if keep is None else keep.shape[0]
+        dalpha_e = dalpha.new_zeros((ctx.rows, dalpha.shape[1]))
+        if keep is None:
+            dalpha_e[:E] = dalpha[:E]
+        else:
+            dalpha_e.index_copy_(0, keep, dalpha[:n_keep])
+        return dalpha_e, dalpha[n_keep:], None, None
+
+
+def attention_weights(alpha_e, alpha_s, keep, E):
+    """PyG GATConv's ``alpha`` [E_nl + N, H] from the per-edge-id ``alpha_e`` [max(E, 1), H] and the loops' ``alpha_s`` [N, H]
+    of ``dcb200::gat_conv_heads``, differentiable; ``keep`` from ``GraphCSR.attention_edges()``, E the number of edges."""
+    return _AttentionWeights.apply(alpha_e, alpha_s, keep, E)
 
 
 def stack_enter(x, edge_index, mode="tag", ptr_host=None):
@@ -1145,15 +1189,25 @@ def gat_aggregate(g, xs, a_src, a_dst, slope, heads, C_, concat, bias=None, relu
     return out, alpha_e, alpha_s
 
 
-def gat_bwd_edge_heads(g, a_src, a_dst, slope, alpha_e, alpha_s, xs, dout, heads, C_, concat):
-    """-> (dz_e [max(E,1), H], dz_s [N, H], da_dst [N, H]); see dc_gat_bwd_edge_heads."""
+def gat_bwd_edge_heads(g, a_src, a_dst, slope, alpha_e, alpha_s, xs, dout, heads, C_, concat, dalpha_e=None, dalpha_s=None):
+    """-> (dz_e [max(E,1), H], dz_s [N, H], da_dst [N, H]); see dc_gat_bwd_edge_heads.  ``dalpha_e`` [max(E,1), H] (by edge id)
+    / ``dalpha_s`` [N, H]: the gradient that reaches alpha itself, added to the one through the aggregation
+    (dc_gat_bwd_edge_heads_ext); without either the call is dc_gat_bwd_edge_heads."""
     hs, scale = _dout_heads(heads, C_, concat)
     dz_e = torch.zeros((max(g.E, 1), heads), dtype=_f32, device=xs.device)
     dz_s = torch.empty((g.N, heads), dtype=_f32, device=xs.device)
     da_dst = torch.empty((g.N, heads), dtype=_f32, device=xs.device)
-    _abi.call("dc_gat_bwd_edge_heads", _ptr(g.rowptr), _ptr(g.nbr), _ptr(g.eid), _ptr(a_src), _ptr(a_dst), float(slope),
-              _ptr(alpha_e), _ptr(alpha_s), _ptr(xs), _rows(xs, "xs"), _ptr(dout), _rows(dout, "dout"), hs, scale, int(heads),
-              int(C_), g.N, _ptr(dz_e), _ptr(dz_s), _ptr(da_dst), _stream())
+    args = (_ptr(g.rowptr), _ptr(g.nbr), _ptr(g.eid), _ptr(a_src), _ptr(a_dst), float(slope), _ptr(alpha_e), _ptr(alpha_s), _ptr(xs),
+            _rows(xs, "xs"), _ptr(dout), _rows(dout, "dout"), hs, scale, int(heads), int(C_), g.N)
+    if dalpha_e is None and dalpha_s is None:
+        _abi.call("dc_gat_bwd_edge_heads", *args, _ptr(dz_e), _ptr(dz_s), _ptr(da_dst), _stream())
+        return dz_e, dz_s, da_dst
+    for t, rows, name in ((dalpha_e, max(g.E, 1), "dalpha_e"), (dalpha_s, g.N, "dalpha_s")):
+        if t is not None:
+            _need(t, _f32, name)
+            if tuple(t.shape) != (rows, heads) or not t.is_contiguous():
+                raise _abi.DcError(f"{name}: expected a contiguous [{rows}, {heads}] tensor, got {tuple(t.shape)}")
+    _abi.call("dc_gat_bwd_edge_heads_ext", *args, _ptr(dalpha_e), _ptr(dalpha_s), _ptr(dz_e), _ptr(dz_s), _ptr(da_dst), _stream())
     return dz_e, dz_s, da_dst
 
 

@@ -493,9 +493,12 @@ def _(x, edge_index, weight, att_src, att_dst, bias, negative_slope, heads, conc
 def gat_conv_heads_backward(dout: Tensor, out: Tensor, x: Tensor, edge_index: Tensor, weight: Tensor, att_src: Tensor,
                             att_dst: Tensor, xs: Tensor, a_src: Tensor, a_dst: Tensor, alpha_e: Tensor, alpha_s: Tensor,
                             negative_slope: float, heads: int, concat: bool, relu: bool, precision: int, ptr: Optional[List[int]],
-                            need_dx: bool, need_db: bool) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
+                            need_dx: bool, need_db: bool, dalpha_e: Optional[Tensor] = None,
+                            dalpha_s: Optional[Tensor] = None) -> Tuple[Tensor, Tensor, Tensor, Tensor, Tensor]:
     """-> (dx, dW, datt_src, datt_dst, dbias); empty tensors for gradients that are not needed.  dz and da_dst by receiver
-    (dc_gat_bwd_edge_heads), then dxs and da_src in one pass by source (dc_gat_scatter_heads), datt by a column reduction."""
+    (dc_gat_bwd_edge_heads), then dxs and da_src in one pass by source (dc_gat_scatter_heads), datt by a column reduction.
+    ``dalpha_e`` [max(E,1), H] / ``dalpha_s`` [N, H]: the gradient of the loss wrt the attention coefficients themselves, added
+    to the one through the aggregation by the receiver pass (dc_gat_bwd_edge_heads_ext); the other passes are unchanged."""
     g = _csr(edge_index, x.shape[0], "gat", ptr)
     dout, db = ops.relu_bwd_db(out, dout.contiguous(), relu, need_db)
     N, Fi = x.shape
@@ -503,7 +506,8 @@ def gat_conv_heads_backward(dout: Tensor, out: Tensor, x: Tensor, edge_index: Te
     C_ = HC // heads
     x = x.contiguous()
     db = db if need_db else dout.new_empty(0)
-    dz_e, dz_s, da_dst = ops.gat_bwd_edge_heads(g, a_src, a_dst, negative_slope, alpha_e, alpha_s, xs, dout, heads, C_, concat)
+    dz_e, dz_s, da_dst = ops.gat_bwd_edge_heads(g, a_src, a_dst, negative_slope, alpha_e, alpha_s, xs, dout, heads, C_, concat,
+                                                dalpha_e, dalpha_s)
     dxs, da_src = ops.gat_scatter_heads(g, alpha_e, alpha_s, dz_e, dz_s, da_dst, att_src, att_dst, dout, heads, C_, concat)
     datt_s, datt_d = ops.gat_att_grad(xs, da_src, da_dst, heads, C_)
     dx = ops.gemm([(dxs, weight)], N, Fi, False, False, precision=precision) if need_dx else dout.new_empty(0)
@@ -513,7 +517,7 @@ def gat_conv_heads_backward(dout: Tensor, out: Tensor, x: Tensor, edge_index: Te
 
 @gat_conv_heads_backward.register_fake
 def _(dout, out, x, edge_index, weight, att_src, att_dst, xs, a_src, a_dst, alpha_e, alpha_s, negative_slope, heads, concat, relu,
-      precision, ptr, need_dx, need_db):
+      precision, ptr, need_dx, need_db, dalpha_e=None, dalpha_s=None):
     return (torch.empty_like(x) if need_dx else x.new_empty(0), torch.empty_like(weight), torch.empty_like(att_src),
             torch.empty_like(att_dst), x.new_empty(dout.shape[1]) if need_db else x.new_empty(0))
 
@@ -526,15 +530,19 @@ def _gat_heads_setup(ctx, inputs, output):
     ctx.set_materialize_grads(False)
 
 
-def _gat_heads_backward(ctx, dout, *_unused):
+def _gat_heads_backward(ctx, dout, _dxs, _da_src, _da_dst, dalpha_e, dalpha_s):
     slope, heads, concat, relu, precision, ptr, has_bias = ctx.meta
     out, x, edge_index, weight, att_src, att_dst, xs, a_src, a_dst, alpha_e, alpha_s = ctx.saved_tensors
-    if dout is None:
+    if dout is None and dalpha_e is None and dalpha_s is None:
         return (None,) * 12
-    need_dx, need_db = ctx.needs_input_grad[0], has_bias and ctx.needs_input_grad[5]
+    need_dx, need_db = ctx.needs_input_grad[0], has_bias and ctx.needs_input_grad[5] and dout is not None
+    if dout is None:
+        dout = torch.zeros_like(out)      # a loss on alpha alone: the kernels read zeros (the bias gets no gradient)
+    dalpha_e = dalpha_e.contiguous() if dalpha_e is not None else None
+    dalpha_s = dalpha_s.contiguous() if dalpha_s is not None else None
     dx, dw, das, dad, db = torch.ops.dcb200.gat_conv_heads_backward(dout, out, x, edge_index, weight, att_src, att_dst, xs, a_src,
                                                                     a_dst, alpha_e, alpha_s, slope, heads, concat, relu, precision,
-                                                                    ptr, need_dx, need_db)
+                                                                    ptr, need_dx, need_db, dalpha_e, dalpha_s)
     return (dx if need_dx else None, None, dw, das, dad, db if need_db else None, None, None, None, None, None, None)
 
 

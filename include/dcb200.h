@@ -415,6 +415,16 @@ DC_API int dc_gat_bwd_edge_heads(const int32_t* rowptr, const int32_t* nbr, cons
                           int64_t ldx, const float* dout, int64_t ldd, int64_t dout_head_stride, float dout_scale,
                           int32_t heads, int32_t C, int64_t num_nodes, float* dz_edge, float* dz_self, float* da_dst,
                           dc_stream_t stream);
+/* dc_gat_bwd_edge_heads for a loss that also reads the attention coefficients (GATConv's return_attention_weights):
+ *   dalpha[e,h] = dout_scale * <dout_h[i], xs_h[src_e]> + dalpha_edge[e,h]  (self loop: + dalpha_self[i,h]),
+ * then the same softmax and leaky-ReLU backward.  dalpha_edge [E, H] by original edge id, dalpha_self [N, H], both row-major
+ * with row stride heads and nullable (null adds nothing; both null runs dc_gat_bwd_edge_heads' kernel, same bits).  dout is
+ * required: a loss on alpha alone passes zeros.  Same checks and outputs as dc_gat_bwd_edge_heads. */
+DC_API int dc_gat_bwd_edge_heads_ext(const int32_t* rowptr, const int32_t* nbr, const int32_t* eid, const float* a_src,
+                              const float* a_dst, float slope, const float* alpha_edge, const float* alpha_self, const float* xs,
+                              int64_t ldx, const float* dout, int64_t ldd, int64_t dout_head_stride, float dout_scale,
+                              int32_t heads, int32_t C, int64_t num_nodes, const float* dalpha_edge, const float* dalpha_self,
+                              float* dz_edge, float* dz_self, float* da_dst, dc_stream_t stream);
 /* Replaces the autograd of the aggregation and of the scores (the transposed propagate and the att products), by source, on the
  * by-source CSR (nbr_t = receivers):  da_src[j,h] = sum_{e: src=j} dz[e,h] + dz_self[j,h];
  *   dxs[j,h,:] = dout_scale (sum_e alpha[e,h] dout_h[dst_e] + alpha_self[j,h] dout_h[j]) + da_src[j,h] att_src[h,:]
