@@ -89,6 +89,37 @@ def measure(C, C64, scale):
     return (ratio.max().item() if C.numel() else 0.0), ij, glob
 
 
+SENTINEL = 0x7FBADBAD          # a NaN payload no kernel writes
+
+
+def sentinel_out(M, N, ld, offset, device="cuda"):
+    """(buffer, C): C [M, N] with row pitch ``ld`` at element ``offset`` of an fp32 buffer filled with the SENTINEL bit pattern,
+    which extends at least one row past C at both ends; ``offset % 4`` is C's distance in floats from a 16-byte boundary."""
+    buf = torch.full((offset + (M + 1) * ld + N,), SENTINEL, dtype=torch.int32, device=device).view(torch.float32)
+    return buf, buf.as_strided((M, N), (ld, 1), offset)
+
+
+def outside_untouched(buf, C, what):
+    """Every element of ``buf`` that is not part of the view ``C`` still holds the sentinel."""
+    mask = torch.ones(buf.shape, dtype=torch.bool, device=buf.device)
+    mask.as_strided(C.shape, C.stride(), C.storage_offset()).fill_(False)
+    assert bool((buf.view(torch.int32)[mask] == SENTINEL).all()), f"{what}: wrote outside C"
+
+
+def epilogue_path(M, N, kb_total, C, bias, accumulate):
+    """The epilogue K2 takes for a single product (gemm_tc2.cu: t2_k_parts, t2_tepi_ok, vec_ok), for the record."""
+    sms = torch.cuda.get_device_properties(C.device).multi_processor_count
+    tiles = -(-M // 128) * -(-N // 128)
+    parts = 1 if tiles >= sms else max(1, min(sms // tiles, kb_total // 8, 64))
+    aligned = C.stride(0) % 4 == 0 and C.data_ptr() % 16 == 0
+    if parts > 1:
+        return "split-k"
+    if not accumulate and aligned and N % 4 == 0:
+        return "tma epilogue"
+    vec = aligned and (bias is None or bias.data_ptr() % 16 == 0)
+    return "staged" if vec else "staged scalar"
+
+
 def check_product(C, C64, scale, tau_elem=TAU_ELEM, tau_global=TAU_GLOBAL, what=""):
     """Assert both bounds; returns (elementwise, global) for the record."""
     elem, (i, j), glob = measure(C, C64, scale)

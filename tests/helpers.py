@@ -63,7 +63,7 @@ def gradient_conditioning(model64, loss_fn, eps=1e-6, samples=3, seed=0):
         m = copy.deepcopy(model64)
         with torch.no_grad():
             for p in m.parameters():
-                p.mul_(1.0 + eps * torch.randn(p.shape, generator=gen, dtype=p.dtype))
+                p.mul_(1.0 + eps * torch.randn(p.shape, generator=gen, dtype=p.dtype).to(p.device))
         m.zero_grad()
         loss_fn(m).backward()
         for k, p in m.named_parameters():

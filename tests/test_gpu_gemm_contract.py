@@ -12,11 +12,10 @@ import collections
 import pytest
 import torch
 
-from gemm_contract import CLASSES, check_product, operands, reference, stored
+from gemm_contract import CLASSES, check_product, epilogue_path, operands, outside_untouched, reference, sentinel_out, stored
 
 pytestmark = pytest.mark.gpu
 
-SENTINEL = 0x7FBADBAD          # a NaN payload no kernel writes
 RECORD = collections.defaultdict(lambda: [0.0, 0.0])
 
 
@@ -46,28 +45,7 @@ def _out(M, N, layout):
     'offset' (C one float past a 16-byte boundary)."""
     Np = (N + 3) // 4 * 4
     width, c0 = {"aligned": (Np + 8, 4), "ldc": (Np + 9, 4), "offset": (Np + 8, 1)}[layout]
-    buf = torch.full((M + 2, width), SENTINEL, dtype=torch.int32, device="cuda").view(torch.float32)
-    return buf, buf[1:1 + M, c0:c0 + N], c0
-
-
-def _outside_untouched(buf, M, N, c0, what):
-    mask = torch.ones(buf.shape, dtype=torch.bool, device=buf.device)
-    mask[1:1 + M, c0:c0 + N] = False
-    assert bool((buf.view(torch.int32)[mask] == SENTINEL).all()), f"{what}: wrote outside C"
-
-
-def _path(M, N, kb_total, C, bias, accumulate):
-    """The epilogue K2 takes for a single product (gemm_tc2.cu: t2_k_parts, t2_tepi_ok, vec_ok), for the record."""
-    sms = torch.cuda.get_device_properties(0).multi_processor_count
-    tiles = -(-M // 128) * -(-N // 128)
-    parts = 1 if tiles >= sms else max(1, min(sms // tiles, kb_total // 8, 64))
-    aligned = C.stride(0) % 4 == 0 and C.data_ptr() % 16 == 0
-    if parts > 1:
-        return "split-k"
-    if not accumulate and aligned and N % 4 == 0:
-        return "tma epilogue"
-    vec = aligned and (bias is None or bias.data_ptr() % 16 == 0)
-    return "staged" if vec else "staged scalar"
+    return sentinel_out(M, N, width, width + c0)
 
 
 def _bias(N, kind, g):
@@ -91,7 +69,7 @@ def _single(dc, M, N, Ks, ta, tb, cls, bias=None, relu=False, accumulate=False, 
     g = torch.Generator(device="cuda").manual_seed(seed + 1)
     b = _bias(N, bias, g)
     c_old = torch.randn(M, N, generator=g, device="cuda") if accumulate else None
-    buf, C, c0 = _out(M, N, out)
+    buf, C = _out(M, N, out)
     what = f"{M}x{N}x{list(Ks)} ta={ta} tb={tb} {cls} bias={bias} relu={relu} acc={accumulate} out={out}"
 
     def run():
@@ -104,9 +82,9 @@ def _single(dc, M, N, Ks, ta, tb, cls, bias=None, relu=False, accumulate=False, 
     C64, scale = reference(segs, ta, tb, bias=b, c_old=c_old, relu=relu)
     kbs = [-(-k // 32) for k in Ks]
     path = "multi-segment " if len(Ks) > 1 else ""
-    path += "chained" if len(Ks) > 4 else _path(M, N, sum(kbs), C, b, accumulate)
+    path += "chained" if len(Ks) > 4 else epilogue_path(M, N, sum(kbs), C, b, accumulate)
     _record(path, cls, C, C64, scale, what)
-    _outside_untouched(buf, M, N, c0, what)
+    outside_untouched(buf, C, what)
     assert torch.equal(first.view(torch.int32), run().view(torch.int32)), f"{what}: second call differs"
     return C.clone()
 
@@ -188,7 +166,7 @@ def _batched(dc, shapes, ta, tb, cls, relu=False, accumulate=False, fused=False,
     for j, (M, N, K) in enumerate(shapes):
         A, B = operands(cls, M, N, K, seed + 7 * j, device="cuda")
         A, B = stored(A, ta), stored(B, tb)
-        buf, C, c0 = _out(M, N, out)
+        buf, C = _out(M, N, out)
         c_old = torch.randn(M, N, generator=g, device="cuda") if accumulate else None
         q = (A, B, C)
         if fused:
@@ -196,15 +174,15 @@ def _batched(dc, shapes, ta, tb, cls, relu=False, accumulate=False, fused=False,
             E = torch.rand((M, ld), generator=g, device="cuda")[:, :N]
             q = q + (E, torch.randn(M, generator=g, device="cuda"))
         probs.append(q)
-        bufs.append((buf, c0, c_old))
+        bufs.append((buf, c_old))
         refs.append(reference([(A, B)], ta, tb, c_old=c_old, E=q[3] if fused else None, rowv=q[4] if fused else None, relu=relu))
 
     def run():
-        for (buf, c0, c_old), q in zip(bufs, probs):
+        for (buf, c_old), q in zip(bufs, probs):
             if c_old is not None:
                 q[2].copy_(c_old)
         ops.gemm_batched(probs, trans_a=ta, trans_b=tb, relu=relu, accumulate=accumulate)
-        return [buf.clone() for buf, _, _ in bufs]
+        return [buf.clone() for buf, _ in bufs]
 
     first = run()
     if fused:
@@ -212,11 +190,11 @@ def _batched(dc, shapes, ta, tb, cls, relu=False, accumulate=False, fused=False,
         path = "batched fused " + ("tma epilogue" if tma else "staged" if out == "aligned" else "staged scalar")
     else:
         path = "batched " + ("staged" if out == "aligned" else "staged scalar")
-    for (M, N, K), q, (C64, scale), (buf, c0, _) in zip(shapes, probs, refs, bufs):
+    for (M, N, K), q, (C64, scale), (buf, _) in zip(shapes, probs, refs, bufs):
         what = f"batched {M}x{N}x{K} ta={ta} tb={tb} {cls} relu={relu} acc={accumulate} fused={fused} out={out} lde+{lde_pad}"
         if M and N:
             _record(path, cls, q[2], C64, scale, what)
-        _outside_untouched(buf, M, N, c0, what)
+        outside_untouched(buf, q[2], what)
     assert all(torch.equal(a.view(torch.int32), b.view(torch.int32)) for a, b in zip(first, run())), "second call differs"
     return [q[2].clone() for q in probs]
 

@@ -40,7 +40,8 @@ def _ref_csr(ei, n, by, drop):
     return rowptr, other[order], eid[order]
 
 
-@pytest.mark.parametrize("n,e", [(1, 0), (5, 0), (7, 20), (1000, 8000), (2049, 2048), (70001, 300017), (300, 100000)])
+@pytest.mark.parametrize("n,e", [(1, 0), (5, 0), (7, 20), (1000, 8000), (2049, 2048), (70001, 300017), (300, 100000),
+                                 (512000, 4096000)])   # last: the C3 step's soft graph (256 x 2000 nodes, kNN-8)
 @pytest.mark.parametrize("by", [0, 1])
 @pytest.mark.parametrize("drop", [False, True])
 def test_csr_build(dc, n, e, by, drop):
@@ -521,7 +522,7 @@ def test_batched_grid_search_bit_identical_to_brute_force(dc):
     """dc_knn_grid_batched / dc_radius_grid_batched (one grid per graph of a batch) == dc_knn / dc_radius (tiled brute force) bit for
     bit, incl. neighbour order and the radius search's truncation to the lowest indices:
     a ragged batch of uniform / clustered / degenerate clouds with an empty graph, a one-point graph and a graph with fewer
-    than k points in between; several k, loop on / off; through ``ptr`` and through a ``batch`` vector; auto dispatch by the
+    than k points in between, and the 256 x 2000 positions of the C3 step; several k, loop on / off; through ``ptr`` and through a ``batch`` vector; auto dispatch by the
     average cloud size; the device-side hand-back of a batch a grid cannot split."""
     from deformcontact_b200 import ops
     g = torch.Generator().manual_seed(5)
@@ -534,8 +535,10 @@ def test_batched_grid_search_bit_identical_to_brute_force(dc):
               clouds["coincident"], torch.rand(5000, 3, generator=g) - 2.0]
     mixed = [clouds["uniform"], tiny[0], clouds["clustered"], tiny[1], clouds["duplicates"], tiny[2], clouds["planar"],
              clouds["lattice"], clouds["coincident"], clouds["shifted"], stretched]
+    # the C3 step's soft graphs: 256 clouds of 2000 points, drawn as synthetic.make_batch draws them
+    c3 = [torch.rand(2000, 3, generator=torch.Generator().manual_seed(1234 + i)) - 0.5 for i in range(256)]
     try:
-        for parts, want_grid in ((benign, True), (mixed, None)):
+        for parts, want_grid in ((benign, True), (mixed, None), (c3, True)):
             sizes = [p.shape[0] for p in parts]
             pos = torch.cat(parts).cuda()
             ptr = torch.tensor([0] + sizes).cumsum(0).cuda()
@@ -656,7 +659,8 @@ def test_staged_hop_chain_unsupported_tile(dc):
     assert _abi.lib().dc_spmm_stage_supported(3500, 128)
 
 
-@pytest.mark.parametrize("M,N", [(1, 1), (5000, 256), (2049, 3), (777, 100), (307300, 256)])   # last: the 128-column float4 blocks
+# (307300, 256): the 128-column float4 blocks; (512000, 256) and (195072, 256): the bias gradients of the C3 step
+@pytest.mark.parametrize("M,N", [(1, 1), (5000, 256), (2049, 3), (777, 100), (307300, 256), (512000, 256), (195072, 256)])
 def test_relu_bwd_colsum_equals_the_two_kernels(dc, M, N):
     """dc_relu_bwd_colsum == dc_relu_bwd followed by dc_colsum, bit for bit (same summation order)."""
     from deformcontact_b200 import ops

@@ -1,6 +1,7 @@
-"""Full-size (BASELINE.json configs) checks through size-independent properties: the oracle is
-too slow at these sizes, so parity is shown by linearity, permutation equivariance, determinism
-and by agreement with an fp64 evaluation on a random sample of rows."""
+"""Full-size (BASELINE.json configs) checks through size-independent properties: linearity, adjointness, permutation
+equivariance, determinism and agreement with an fp64 evaluation on a random sample of rows.  These complement, not replace,
+oracle parity at full size: run on the GPU, the oracle is fast enough at C3 (tests/test_gpu_c3_shapes.py compares the step,
+its K1 hops and its K2 products with it there)."""
 import pytest
 import torch
 
